@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — path segments/sec of the B200-native ray_color bounce loop (see BASELINE.json / BASELINE.md).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload C1|C2|C3|C4|C5] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload C1|C2|C3|C4|C5] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one full render of the workload (every pixel, `spp` samples) on each rank.  N > 1 is launched by
 torchrun (one process per GPU): rank r renders global samples [r*spp, (r+1)*spp) of every pixel (WEAK scaling: per-GPU
@@ -15,6 +15,8 @@ total spp (--strong-spp, stated) SPLIT across the ranks, 133 MB reduce — so th
           H2D), render, reduce, D2H of the accumulation buffer — every step.
 `--impl reference` times the reference's CPU algorithm (the f64 oracle port: the Rust reference cannot be compiled in
 this image) on all host cores, on a bounded sample (1 spp at full resolution per step) of the same workload.
+`--dump-outputs DIR` writes what the last timed step computed (rank 0's accumulation buffer and its path counters) as
+.npy files, so that two builds can be compared output for output on the same seeded workload.
 """
 import argparse
 import json
@@ -130,6 +132,25 @@ def measured_peaks():
     return {"hbm_gbs": 6650.0, "sm_max_mhz": 1965.0}, "fallback"
 
 
+DUMP_BYTES = 64 << 20
+DUMP_SAMPLE_PIXELS = 1 << 21
+
+
+def dump_outputs(out_dir, accum, st):
+    """Writes the last timed step's outputs: accum.npy, the (H, W, 4) float32 sums of R, G, B, Y^2 per pixel, and
+    counters.npy, float64 [paths, segments, rejected].  A buffer over DUMP_BYTES is cut to a fixed seeded sample of
+    DUMP_SAMPLE_PIXELS pixels, (n, 4) float32, whose row-major pixel indices go to accum_pixel_index.npy (float64)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    if accum.nbytes > DUMP_BYTES:
+        h, w, _ = accum.shape
+        idx = np.sort(np.random.default_rng(0).choice(h * w, DUMP_SAMPLE_PIXELS, replace=False))
+        np.save(os.path.join(out_dir, "accum_pixel_index.npy"), idx.astype(np.float64))
+        accum = accum.reshape(-1, 4)[idx]
+    np.save(os.path.join(out_dir, "accum.npy"), accum)
+    np.save(os.path.join(out_dir, "counters.npy"), np.array([st["paths"], st["segments"], st["rejected"]], dtype=np.float64))
+
+
 def run_reference(args, rank):
     """The reference's CPU implementation of the path (oracle port, all host threads), bounded sample per step."""
     if rank != 0:
@@ -176,7 +197,11 @@ def main():
                          "rendered by every rank (weak, default)")
     ap.add_argument("--strong-spp", type=int, default=2048,
                     help="total spp of the C5 strong-scaling sub-record (split across the ranks); 0 = skip it")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's accumulation buffer and path counters to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -263,6 +288,8 @@ def main():
         launches += st["launches"]
     e1.record(stream)
     barrier()
+    if args.dump_outputs and rank == 0:  # before the e2e and roofline renders below overwrite the buffer
+        dump_outputs(args.dump_outputs, accum.cpu().numpy(), st)
     ms = e0.elapsed_time(e1)
     reduce_ms = sum(reduce_ms_list) / max(len(reduce_ms_list), 1)
     wait_ms = sum(wait_ms_list) / max(len(wait_ms_list), 1)

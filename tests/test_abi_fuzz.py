@@ -3,12 +3,14 @@
 (including cycles), material / texture / table ids, parameters set to NaN / inf / huge / negative, truncated arrays — and
 pushed through rtb_scene_set_* + rtb_scene_build_bvh in a host-only scene.  Run in a subprocess so that a crash is a
 test failure, not the end of the test session."""
+import os
 import subprocess
 import sys
 import textwrap
 
 import pytest
 
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))  # the child script imports from here and from tests/
 SCRIPT = textwrap.dedent(r'''
     import sys, copy
     import numpy as np
@@ -75,7 +77,8 @@ SCRIPT = textwrap.dedent(r'''
 
 @pytest.mark.parametrize("chunk", [0, 1, 2])
 def test_corrupted_scene_records_never_crash(chunk):
-    r = subprocess.run([sys.executable, "-c", SCRIPT, str(20 * chunk), str(20 * chunk + 20)], capture_output=True, text=True, timeout=900)
+    r = subprocess.run([sys.executable, "-c", SCRIPT, str(20 * chunk), str(20 * chunk + 20)], capture_output=True, text=True, timeout=900,
+                       cwd=ROOT)
     assert r.returncode == 0, f"exit code {r.returncode}\n{r.stdout[-2000:]}\n{r.stderr[-3000:]}"
     assert "outcomes" in r.stdout
     print(r.stdout.strip().splitlines()[-1])
@@ -85,6 +88,6 @@ def test_corrupted_scene_records_never_crash(chunk):
 def test_corrupted_scenes_render_or_are_refused():
     """GPU tier: every corrupted scene the host accepts (parameters that are finite but absurd, odd but legal wiring) is
     rendered at 32x24x4 — the device must finish and account for every path."""
-    r = subprocess.run([sys.executable, "-c", SCRIPT, "0", "40", "gpu"], capture_output=True, text=True, timeout=600)
+    r = subprocess.run([sys.executable, "-c", SCRIPT, "0", "40", "gpu"], capture_output=True, text=True, timeout=600, cwd=ROOT)
     assert r.returncode == 0, f"exit code {r.returncode}\n{r.stdout[-2000:]}\n{r.stderr[-3000:]}"
     print(r.stdout.strip().splitlines()[-1])
