@@ -207,6 +207,50 @@ __device__ __forceinline__ float sqrt_fast(float x) {
 #endif
 }
 
+// Packed FP32 pairs (sm_100 FFMA2 / FADD2 / FMUL2: two lanes of the FMA pipe in ONE issued instruction).  Each element is
+// the scalar IEEE round-to-nearest operation (no .ftz: the library is built without fast-math), so a pair of results is
+// bit for bit what two scalar instructions give.  Inline PTX keeps the compiler from contracting an add into a
+// neighbouring multiply or splitting the pair; a float2 whose halves are equal (make_float2(s, s)) becomes a broadcast
+// operand, no register copy.  The host build (tests/emul) uses the scalar operations.
+#ifdef __CUDA_ARCH__
+__device__ __forceinline__ unsigned long long pk2(float2 a) {
+  unsigned long long r;
+  asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(a.x), "f"(a.y));
+  return r;
+}
+__device__ __forceinline__ float2 upk2(unsigned long long r) {
+  float2 a;
+  asm("mov.b64 {%0, %1}, %2;" : "=f"(a.x), "=f"(a.y) : "l"(r));
+  return a;
+}
+__device__ __forceinline__ float2 ffma2(float2 a, float2 b, float2 c) {  // a * b + c, one rounding per element
+  unsigned long long r;
+  asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(r) : "l"(pk2(a)), "l"(pk2(b)), "l"(pk2(c)));
+  return upk2(r);
+}
+__device__ __forceinline__ float2 fadd2(float2 a, float2 b) {
+  unsigned long long r;
+  asm("add.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(pk2(a)), "l"(pk2(b)));
+  return upk2(r);
+}
+__device__ __forceinline__ float2 fsub2(float2 a, float2 b) {
+  unsigned long long r;
+  asm("sub.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(pk2(a)), "l"(pk2(b)));
+  return upk2(r);
+}
+__device__ __forceinline__ float2 fmul2(float2 a, float2 b) {
+  unsigned long long r;
+  asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(pk2(a)), "l"(pk2(b)));
+  return upk2(r);
+}
+#else
+__device__ __forceinline__ float2 ffma2(float2 a, float2 b, float2 c) { return make_float2(fmaf(a.x, b.x, c.x), fmaf(a.y, b.y, c.y)); }
+__device__ __forceinline__ float2 fadd2(float2 a, float2 b) { return make_float2(a.x + b.x, a.y + b.y); }
+__device__ __forceinline__ float2 fsub2(float2 a, float2 b) { return make_float2(a.x - b.x, a.y - b.y); }
+__device__ __forceinline__ float2 fmul2(float2 a, float2 b) { return make_float2(a.x * b.x, a.y * b.y); }
+#endif
+__device__ __forceinline__ float2 f2s(float s) { return make_float2(s, s); }  // broadcast
+
 // ---- Philox4x32-10: key = (pixel, sample), counter = (block, bounce, seed, 'RTB2').  Replaces rand::random
 // (rt_weekend.rs:8-19); identical to oracle/rt_oracle.hpp so streams can be compared draw by draw.
 enum RngBlock : uint32_t { BLK_CAMERA0 = 0, BLK_CAMERA1 = 1, BLK_SCATTER = 2, BLK_AUX = 3, BLK_MEDIUM0 = 8 };
@@ -663,6 +707,17 @@ struct Trav {
   Closest best;
   float amb;        // ambiguity horizon: smallest distance at which an undecided candidate may lie (inf = none)
 };
+// slot mask -> priority mask of a ray with octant word `octinv` (bit p of the result = bit p ^ octinv of `m`)
+__device__ __forceinline__ uint32_t octant_remap(uint32_t m, uint32_t octinv) {
+  if (octinv & 1u) m = ((m & 0x55u) << 1) | ((m & 0xAAu) >> 1);
+  if (octinv & 2u) m = ((m & 0x33u) << 2) | ((m & 0xCCu) >> 2);
+  if (octinv & 4u) m = ((m & 0x0Fu) << 4) | ((m & 0xF0u) >> 4);
+  return m;
+}
+// octant_remap() of every (octinv, 8-bit mask) as a 2 KB table in shared memory, for the fully staged static kernels:
+// one LDS.U8 per node visit (table base in a uniform register) instead of the three conditional swaps (~12 ALU-pipe
+// instructions).  The kernel fills it (octmap_fill(), rtb_kernels.cu) before its first __syncthreads().
+__shared__ uint8_t s_octmap[8 * 256];
 // the ray must be re-traced exactly: something undecided may lie at or before the closest certain hit
 __device__ __forceinline__ bool needs_exact(const Closest& best, float amb) { return amb < INFINITY && amb <= best.hi; }
 // what k_fixup has to do for a finished ray: 0 nothing, 1 exact re-trace, 2 recompute the distance of its (certain) hit
@@ -768,7 +823,11 @@ __device__ __forceinline__ void expand_leaves(uint32_t leaf, uint32_t w1y, uint3
 // (intersect_prim) or park them to test many lanes' primitives together; the exact pass runs exact_hit on them.
 // STRIDE: distance (in entries) between consecutive levels of the ray's stack (1 = a private array; the warp-queue kernel
 // keeps the stacks of a warp's rays interleaved in shared memory).
-template <bool COUNT, bool ALL_STAGED, int STRIDE = 1, class Leaves>
+// PACKED: the child slab test on packed FP32 pairs (FFMA2 / FADD2); the same bits as the scalar form, fewer instructions.
+// Used by the fully staged static kernels (C1 / C2); the others keep the scalar form, which measured as fast or faster
+// there (the deep-tree kernels' register allocation: C4 -1 % packed).
+// OCTMAP: the hit mask's octant remap through the shared-memory table (the kernel fills it, see octmap_fill()).
+template <bool COUNT, bool ALL_STAGED, int STRIDE = 1, bool PACKED = false, bool OCTMAP = false, class Leaves>
 __device__ __forceinline__ bool trav_step(const DevScene& sc, const uint4* __restrict__ snodes, uint32_t sbase, uint32_t n_snodes,
                                           Trav& tv, uint2* __restrict__ stack, float tmin,
                                           uint32_t& n_nodes_visited, Leaves&& leaves_fn) {
@@ -817,26 +876,52 @@ __device__ __forceinline__ bool trav_step(const DevScene& sc, const uint4* __res
   const uint32_t ny0 = ny ? w4.x : w2.z, ny1 = ny ? w4.y : w2.w, fy0 = ny ? w2.z : w4.x, fy1 = ny ? w2.w : w4.y;
   const uint32_t nz0 = nz ? w4.z : w3.x, nz1 = nz ? w4.w : w3.y, fz0 = nz ? w3.x : w4.z, fz1 = nz ? w3.y : w4.w;
   // child i is hit iff max(tn_xyz, tmin) <= min(tf_xyz, t_max)  <=>  tn3 <= tf3  and  tn3 <= t_max  and  tmin <= tf3
-  // (tmin <= t_max always).  The three differences are FADDs (FMA pipe); their sign bits are OR-ed with one LOP3 and
+  // (tmin <= t_max always).  The three differences are on the FMA pipe; their sign bits are OR-ed with one LOP3 and
   // shifted into the mask with one funnel shift: 4 ALU-pipe instructions per child (2 FMNMX3, LOP3, SHF) instead of
   // 6.4 (2 FMNMX, 2 FMNMX3, FSETP, SEL, IADD3/3) — the node test is ALU-pipe bound (profiles/r1d_c1_ncu_summary.md).
-  uint32_t missmask = 0;
   const uint32_t magic = sc.prmt_magic;  // 0x43000000, read from the constant bank (ptxas cannot fold it into the PRMT)
   const float tmax = tv.best.hi;  // upper bound of the closest hit's exact distance: a subtree is culled only if it
                                   // cannot hold a hit at or before it (equal t must still reach the id tie-break)
+  uint32_t missmask;
+  if constexpr (PACKED) {
+    // Children i and i + 4 read their plane bytes from the same byte of the 0-3 / 4-7 words and share scale and bias:
+    // each plane of the pair is one FFMA2 (the two PRMTs write an aligned register pair), and tf - tn one FADD2.  The
+    // min / max (no packed form), the two differences against the ray's bounds and the sign-bit assembly stay per child
+    // (packing those too costs the 80-register kernels spills).  Every element is the scalar operation, bit for bit.
+    uint32_t mlo = 0, mhi = 0;  // miss bits of children 0-3 | 4-7
 #pragma unroll
-  for (int i = 7; i >= 0; --i) {
-    const uint32_t sel = 0x7044u | ((uint32_t)(i & 3) << 8);
-    const float tnx = fmaf(q2f(i < 4 ? nx0 : nx1, magic, sel), ax, bnx);
-    const float tny = fmaf(q2f(i < 4 ? ny0 : ny1, magic, sel), ay, bny);
-    const float tnz = fmaf(q2f(i < 4 ? nz0 : nz1, magic, sel), az, bnz);
-    const float tfx = fmaf(q2f(i < 4 ? fx0 : fx1, magic, sel), ax, bfx);
-    const float tfy = fmaf(q2f(i < 4 ? fy0 : fy1, magic, sel), ay, bfy);
-    const float tfz = fmaf(q2f(i < 4 ? fz0 : fz1, magic, sel), az, bfz);
-    const float tn = fmaxf(fmaxf(tnx, tny), tnz);
-    const float tf = fminf(fminf(tfx, tfy), tfz);
-    const uint32_t neg = __float_as_uint(tf - tn) | __float_as_uint(tmax - tn) | __float_as_uint(tf - tmin);
-    missmask = __funnelshift_l(neg, missmask, 1);  // (missmask << 1) | sign bit; child 0 ends in bit 0
+    for (int i = 3; i >= 0; --i) {
+      const uint32_t sel = 0x7044u | ((uint32_t)i << 8);
+      const float2 tnx = ffma2(make_float2(q2f(nx0, magic, sel), q2f(nx1, magic, sel)), f2s(ax), f2s(bnx));
+      const float2 tny = ffma2(make_float2(q2f(ny0, magic, sel), q2f(ny1, magic, sel)), f2s(ay), f2s(bny));
+      const float2 tnz = ffma2(make_float2(q2f(nz0, magic, sel), q2f(nz1, magic, sel)), f2s(az), f2s(bnz));
+      const float2 tfx = ffma2(make_float2(q2f(fx0, magic, sel), q2f(fx1, magic, sel)), f2s(ax), f2s(bfx));
+      const float2 tfy = ffma2(make_float2(q2f(fy0, magic, sel), q2f(fy1, magic, sel)), f2s(ay), f2s(bfy));
+      const float2 tfz = ffma2(make_float2(q2f(fz0, magic, sel), q2f(fz1, magic, sel)), f2s(az), f2s(bfz));
+      const float2 tn = make_float2(fmaxf(fmaxf(tnx.x, tny.x), tnz.x), fmaxf(fmaxf(tnx.y, tny.y), tnz.y));
+      const float2 tf = make_float2(fminf(fminf(tfx.x, tfy.x), tfz.x), fminf(fminf(tfx.y, tfy.y), tfz.y));
+      const float2 d = fsub2(tf, tn);
+      // (m << 1) | sign bit: child i ends in bit i of its half
+      mlo = __funnelshift_l(__float_as_uint(d.x) | __float_as_uint(tmax - tn.x) | __float_as_uint(tf.x - tmin), mlo, 1);
+      mhi = __funnelshift_l(__float_as_uint(d.y) | __float_as_uint(tmax - tn.y) | __float_as_uint(tf.y - tmin), mhi, 1);
+    }
+    missmask = (mhi << 4) | mlo;
+  } else {
+    missmask = 0;
+#pragma unroll
+    for (int i = 7; i >= 0; --i) {
+      const uint32_t sel = 0x7044u | ((uint32_t)(i & 3) << 8);
+      const float tnx = fmaf(q2f(i < 4 ? nx0 : nx1, magic, sel), ax, bnx);
+      const float tny = fmaf(q2f(i < 4 ? ny0 : ny1, magic, sel), ay, bny);
+      const float tnz = fmaf(q2f(i < 4 ? nz0 : nz1, magic, sel), az, bnz);
+      const float tfx = fmaf(q2f(i < 4 ? fx0 : fx1, magic, sel), ax, bfx);
+      const float tfy = fmaf(q2f(i < 4 ? fy0 : fy1, magic, sel), ay, bfy);
+      const float tfz = fmaf(q2f(i < 4 ? fz0 : fz1, magic, sel), az, bfz);
+      const float tn = fmaxf(fmaxf(tnx, tny), tnz);
+      const float tf = fminf(fminf(tfx, tfy), tfz);
+      const uint32_t neg = __float_as_uint(tf - tn) | __float_as_uint(tmax - tn) | __float_as_uint(tf - tmin);
+      missmask = __funnelshift_l(neg, missmask, 1);  // (missmask << 1) | sign bit; child 0 ends in bit 0
+    }
   }
   const uint32_t hitmask = ~missmask & 0xFFu;
 #if !defined(__CUDA_ARCH__) && defined(RTB_EMUL_STATS)
@@ -847,9 +932,8 @@ __device__ __forceinline__ bool trav_step(const DevScene& sc, const uint4* __res
 #endif
   // internal children: slot mask -> priority mask (bit p = slot ^ octinv)
   uint32_t ih = hitmask & imask;
-  if (octinv & 1u) ih = ((ih & 0x55u) << 1) | ((ih & 0xAAu) >> 1);
-  if (octinv & 2u) ih = ((ih & 0x33u) << 2) | ((ih & 0xCCu) >> 2);
-  if (octinv & 4u) ih = ((ih & 0x0Fu) << 4) | ((ih & 0xF0u) >> 4);
+  if constexpr (OCTMAP) ih = s_octmap[(octinv << 8) | ih];  // one shared-memory byte instead of three conditional swaps
+  else ih = octant_remap(ih, octinv);
   tv.grp = make_uint2(w1.x, (ih << 8) | imask);
   // (measured and removed: prefetching the next step's node into L1 here, -4 % — and even switched off the dormant path
   //  cost the deep-tree kernels 2-3 %, profiles/r3_ab.md §3)
@@ -880,11 +964,11 @@ __device__ __forceinline__ void trav_globals(const DevScene& sc, Trav& tv, float
 }
 
 // one hot-path step: the leaf primitives go through the f32 tests
-template <bool COUNT, bool ALL_STAGED = false>
+template <bool COUNT, bool ALL_STAGED = false, bool PACKED = false, bool OCTMAP = false>
 __device__ __forceinline__ bool trav_step_fast(const DevScene& sc, const uint4* __restrict__ snodes, uint32_t sbase, uint32_t n_snodes,
                                                Trav& tv, uint2* __restrict__ stack, float tmin,
                                                uint32_t& n_nodes_visited, TestCount& n_tests) {
-  return trav_step<COUNT, ALL_STAGED>(sc, snodes, sbase, n_snodes, tv, stack, tmin, n_nodes_visited,
+  return trav_step<COUNT, ALL_STAGED, 1, PACKED, OCTMAP>(sc, snodes, sbase, n_snodes, tv, stack, tmin, n_nodes_visited,
                                       [&](uint32_t leaf, uint32_t w1y, uint32_t w1z, uint32_t w1w) {
                                         expand_leaves(leaf, w1y, w1z, w1w, [&](uint32_t type, uint32_t idx) {
                                           intersect_prim<COUNT>(sc, type, idx, tv.o, tv.d, tv.time, tmin, tv.best, tv.amb, tv.octinv, n_tests);
@@ -897,12 +981,13 @@ __device__ __forceinline__ bool trav_step_fast(const DevScene& sc, const uint4* 
 // drains: all parked lanes test their primitives TOGETHER, one primitive type at a time, one primitive per iteration.
 // The per-ray order of node visits and primitive tests is unchanged, so results, counters and the exact-pass set are
 // identical to the inline form; only how many lanes execute a primitive test at once changes (inline: the ~1/3 of the
-// lanes whose node happened to have a leaf hit; drained: >= the threshold).
+// lanes whose node happened to have a leaf hit; drained: >= the threshold).  Used by the 64-register dynamic-fetch kernel,
+// with the scalar slab test (the packed one spills there).
 template <bool COUNT, bool ALL_STAGED = false>
 __device__ __forceinline__ bool trav_step_park(const DevScene& sc, const uint4* __restrict__ snodes, uint32_t sbase, uint32_t n_snodes,
                                                Trav& tv, uint2* __restrict__ stack, float tmin, uint32_t& n_nodes_visited,
                                                uint4* __restrict__ park, bool& parked) {
-  return trav_step<COUNT, ALL_STAGED>(sc, snodes, sbase, n_snodes, tv, stack, tmin, n_nodes_visited,
+  return trav_step<COUNT, ALL_STAGED, 1, false>(sc, snodes, sbase, n_snodes, tv, stack, tmin, n_nodes_visited,
                                       [&](uint32_t leaf, uint32_t w1y, uint32_t w1z, uint32_t w1w) {
                                         *park = make_uint4(leaf, w1y, w1z, w1w);
                                         parked = true;
@@ -928,7 +1013,7 @@ __device__ __forceinline__ void drain_parked(const DevScene& sc, Trav& tv, float
 }
 
 // returns the ray's FixKind
-template <bool COUNT, bool ALL_STAGED = false>
+template <bool COUNT, bool ALL_STAGED = false, bool PACKED = false, bool OCTMAP = false>
 __device__ __forceinline__ uint32_t traverse(const DevScene& sc, const uint4* __restrict__ snodes, uint32_t sbase, uint32_t n_snodes,
                                          float3 o, float3 d, float time, float tmin, Closest& best, float& slab_lo_out,
                                          uint32_t& n_nodes_visited, TestCount& n_tests) {
@@ -936,7 +1021,7 @@ __device__ __forceinline__ uint32_t traverse(const DevScene& sc, const uint4* __
   uint2 stack[RTB_STACK];
   trav_init(tv, o, d, time);
   trav_globals<COUNT>(sc, tv, tmin, n_tests);
-  while (trav_step_fast<COUNT, ALL_STAGED>(sc, snodes, sbase, n_snodes, tv, stack, tmin, n_nodes_visited, n_tests)) {}
+  while (trav_step_fast<COUNT, ALL_STAGED, PACKED, OCTMAP>(sc, snodes, sbase, n_snodes, tv, stack, tmin, n_nodes_visited, n_tests)) {}
   best = tv.best;
   slab_lo_out = slab_lo(tv);
   return fix_kind(sc, tv);

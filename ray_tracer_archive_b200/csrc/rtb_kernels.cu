@@ -53,6 +53,11 @@ __device__ __forceinline__ void stage_nodes(const DevScene& sc, uint4* snodes, u
   __syncthreads();
 }
 
+// the octant remap table of trav_step<..., OCTMAP = true> (rtb_device.cuh), filled before stage_nodes()' barrier
+__device__ __forceinline__ void octmap_fill() {
+  for (uint32_t i = threadIdx.x; i < 8u * 256u; i += blockDim.x) s_octmap[i] = (uint8_t)octant_remap(i & 0xFFu, i >> 8);
+}
+
 // media + classification + result write of one finished ray (Material trait dispatch, material.rs:11-21): the info word
 // carries material | face mode | shade queue, resolved on the host, so no material fetch is needed here
 __device__ __forceinline__ void finish_ray(const DevScene& sc, const DevPool& pool, const DevParams& prm, uint32_t slot,
@@ -657,6 +662,7 @@ k_extend_static(DevScene sc, DevPool pool, DevParams prm, uint32_t n_snodes) {
   __shared__ uint8_t s_list[RTB_EXTEND_WARPS][RTB_CHUNK];
   __shared__ uint32_t s_cnt[SORT ? RTB_EXTEND_WARPS : 1][64];
   DevCounters* c = pool.c;
+  if constexpr (ALL_STAGED) octmap_fill();
   stage_nodes(sc, snodes, n_snodes);
   uint32_t sbase = (uint32_t)__cvta_generic_to_shared(snodes);
   asm volatile("mov.u32 %0, %0;" : "+r"(sbase));  // opaque: keep it in a register instead of re-deriving it per node visit
@@ -677,7 +683,9 @@ k_extend_static(DevScene sc, DevPool pool, DevParams prm, uint32_t n_snodes) {
         const float4 rd = pool.ray[2 * slot + 1];
         Closest best;
         float lo;
-        const uint32_t fix = traverse<COUNT, ALL_STAGED>(sc, snodes, sbase, n_snodes, xyz(ro), xyz(rd), ro.w, RTB_TMIN, best, lo, nv, nt);
+        // packed slab test and remap table in the fully staged production kernel (the counting build keeps the scalar
+        // test: same decisions, and the packed one spills there)
+        const uint32_t fix = traverse<COUNT, ALL_STAGED, ALL_STAGED && !COUNT, ALL_STAGED>(sc, snodes, sbase, n_snodes, xyz(ro), xyz(rd), ro.w, RTB_TMIN, best, lo, nv, nt);
         finish_ray(sc, pool, prm, slot, xyz(ro), xyz(rd), best);
         if (fix) queue_fix(pool, slot, fix, lo, best.hi);
       }
