@@ -751,7 +751,7 @@ static int upload_scene(rtb_scene* s, const rtb_scene* host) {
   CU(s->d_self.resize(1));
   d.self = s->d_self.p;
   CU(cudaMemcpy(s->d_self.p, &d, sizeof(DevScene), cudaMemcpyHostToDevice));  // (after every other field is final)
-  int e = configure_launch(s->lc, d.n_nodes, s->bvh.max_depth, s->ctx->prop.multiProcessorCount);
+  int e = configure_launch(s->lc, d.n_nodes, s->bvh.max_depth, d.n_prims[PT_SPHERE], s->ctx->prop.multiProcessorCount);
   if (e != 0) return set_err(RTB_ERR_CUDA, std::string("configure_launch: ") + cudaGetErrorString((cudaError_t)e));
   CU(cudaStreamSynchronize(0));
   s->committed = true;

@@ -801,6 +801,17 @@ __device__ __forceinline__ uint4 lds_node_word(const uint4* __restrict__ snodes,
   return snodes[5 * node + w];
 #endif
 }
+// sphere record `idx` from the shared-memory copy of the sphere array (the fully staged production kernel stages it after
+// the nodes; `ssph` = its 32-bit shared address, kept in a register like `sbase`).  The host build reads the scene's array.
+__device__ __forceinline__ float4 lds_sphere(const DevScene& sc, uint32_t ssph, uint32_t idx) {
+#ifdef __CUDA_ARCH__
+  float4 r;
+  asm("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "r"(ssph + idx * 16u));
+  return r;
+#else
+  return sc.geom[PT_SPHERE][idx];
+#endif
+}
 
 // returns false when the traversal is complete.  ALL_STAGED: every node of the tree is in the shared-memory stage (small
 // scenes), so the global-memory fetch path and its five predicated loads + register moves are compiled out.
@@ -929,6 +940,13 @@ __device__ __forceinline__ bool trav_step(const DevScene& sc, const uint4* __res
   if (!hitmask) ++g_emul_stats[1];      // ... that found no child to continue with (stale stack entries, loose boxes)
   g_emul_stats[2] += __builtin_popcount(hitmask & imask);   // internal children hit
   g_emul_stats[3] += __builtin_popcount(hitmask & ~imask);  // leaf children hit
+  {  // visits whose hit leaves hold 1 / 2 / 3+ primitives (the trips of the leaf loop)
+    uint32_t np = 0;
+    for (uint32_t s = 0; s < 8; ++s)
+      if ((hitmask & ~imask) >> s & 1u) np += (((s < 4 ? w1.z : w1.w) >> (8 * (s & 3))) & 0xFFu) >> 5;
+    if (np) ++g_emul_stats[np == 1 ? 4 : (np == 2 ? 5 : 6)];
+    g_emul_stats[7] += np;
+  }
 #endif
   // internal children: slot mask -> priority mask (bit p = slot ^ octinv)
   uint32_t ih = hitmask & imask;
@@ -964,14 +982,26 @@ __device__ __forceinline__ void trav_globals(const DevScene& sc, Trav& tv, float
 }
 
 // one hot-path step: the leaf primitives go through the f32 tests
-template <bool COUNT, bool ALL_STAGED = false, bool PACKED = false, bool OCTMAP = false>
+// SPHSTAGE: sphere records come from the shared-memory copy at `ssph` (lds_sphere: one LDS.128 through a register address)
+// instead of a read-only global load; the test itself is prim_test()'s sphere_fast(), so the results are the same bits.
+template <bool COUNT, bool ALL_STAGED = false, bool PACKED = false, bool OCTMAP = false, bool SPHSTAGE = false>
 __device__ __forceinline__ bool trav_step_fast(const DevScene& sc, const uint4* __restrict__ snodes, uint32_t sbase, uint32_t n_snodes,
                                                Trav& tv, uint2* __restrict__ stack, float tmin,
-                                               uint32_t& n_nodes_visited, TestCount& n_tests) {
+                                               uint32_t& n_nodes_visited, TestCount& n_tests, uint32_t ssph = 0u) {
   return trav_step<COUNT, ALL_STAGED, 1, PACKED, OCTMAP>(sc, snodes, sbase, n_snodes, tv, stack, tmin, n_nodes_visited,
                                       [&](uint32_t leaf, uint32_t w1y, uint32_t w1z, uint32_t w1w) {
                                         expand_leaves(leaf, w1y, w1z, w1w, [&](uint32_t type, uint32_t idx) {
-                                          intersect_prim<COUNT>(sc, type, idx, tv.o, tv.d, tv.time, tmin, tv.best, tv.amb, tv.octinv, n_tests);
+                                          if (SPHSTAGE && type == PT_SPHERE) {
+                                            if (COUNT) ++n_tests.n[PT_SPHERE];
+                                            RTB_CHECK(CHK_PRIM, idx < sc.n_prims[PT_SPHERE]);
+                                            float t, e = 0.0f;
+                                            bool coarse = false;
+                                            const float4 s = lds_sphere(sc, ssph, idx);
+                                            const int st = sphere_fast(tv.o, tv.d, xyz(s), s.w, tmin, tv.best.hi, t, e, coarse);
+                                            apply_result(tv.best, tv.amb, tv.octinv, st, t, e, ((uint32_t)PT_SPHERE << REF_TYPE_SHIFT) | idx, coarse);
+                                          } else {
+                                            intersect_prim<COUNT>(sc, type, idx, tv.o, tv.d, tv.time, tmin, tv.best, tv.amb, tv.octinv, n_tests);
+                                          }
                                         });
                                       });
 }
@@ -1013,15 +1043,15 @@ __device__ __forceinline__ void drain_parked(const DevScene& sc, Trav& tv, float
 }
 
 // returns the ray's FixKind
-template <bool COUNT, bool ALL_STAGED = false, bool PACKED = false, bool OCTMAP = false>
+template <bool COUNT, bool ALL_STAGED = false, bool PACKED = false, bool OCTMAP = false, bool SPHSTAGE = false>
 __device__ __forceinline__ uint32_t traverse(const DevScene& sc, const uint4* __restrict__ snodes, uint32_t sbase, uint32_t n_snodes,
                                          float3 o, float3 d, float time, float tmin, Closest& best, float& slab_lo_out,
-                                         uint32_t& n_nodes_visited, TestCount& n_tests) {
+                                         uint32_t& n_nodes_visited, TestCount& n_tests, uint32_t ssph = 0u) {
   Trav tv;
   uint2 stack[RTB_STACK];
   trav_init(tv, o, d, time);
   trav_globals<COUNT>(sc, tv, tmin, n_tests);
-  while (trav_step_fast<COUNT, ALL_STAGED, PACKED, OCTMAP>(sc, snodes, sbase, n_snodes, tv, stack, tmin, n_nodes_visited, n_tests)) {}
+  while (trav_step_fast<COUNT, ALL_STAGED, PACKED, OCTMAP, SPHSTAGE>(sc, snodes, sbase, n_snodes, tv, stack, tmin, n_nodes_visited, n_tests, ssph)) {}
   best = tv.best;
   slab_lo_out = slab_lo(tv);
   return fix_kind(sc, tv);

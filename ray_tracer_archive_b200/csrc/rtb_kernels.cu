@@ -655,14 +655,21 @@ k_extend_wq(DevScene sc, DevPool pool, DevParams prm, uint32_t n_snodes) {
 // stage: C3 +6 %; fully staged trees lose 3 %, the dynamic kernel is indifferent — profiles/r3_ab.md §4).  Parking the
 // leaf tests (as the dynamic kernel does) costs this kernel 13 %: with one ray per thread the lanes that wait for a drain
 // are simply idle.  Both are compile-time choices so that each variant's loop carries only its own path.
-template <bool COUNT, bool ALL_STAGED, bool SORT>
+// SPHSTAGE (fully staged trees whose sphere array fits RTB_SPHERE_STAGE_BYTES, configure_launch): the sphere records are
+// staged in shared memory after the nodes and the leaf tests read them from there (trav_step_fast).
+template <bool COUNT, bool ALL_STAGED, bool SORT, bool SPHSTAGE = false>
 __global__ void __maxnreg__(RTB_EXTEND_MAXREG)
 k_extend_static(DevScene sc, DevPool pool, DevParams prm, uint32_t n_snodes) {
+  static_assert(!SPHSTAGE || (ALL_STAGED && !COUNT), "the sphere stage is built for the fully staged production kernel");
   extern __shared__ uint4 snodes[];
   __shared__ uint8_t s_list[RTB_EXTEND_WARPS][RTB_CHUNK];
   __shared__ uint32_t s_cnt[SORT ? RTB_EXTEND_WARPS : 1][64];
   DevCounters* c = pool.c;
   if constexpr (ALL_STAGED) octmap_fill();
+  if constexpr (SPHSTAGE) {  // the sphere array right after the nodes (float4 records = 16-byte words), before stage_nodes()' barrier
+    const uint4* sph = reinterpret_cast<const uint4*>(sc.geom[PT_SPHERE]);
+    for (uint32_t i = threadIdx.x; i < sc.n_prims[PT_SPHERE]; i += blockDim.x) snodes[5u * n_snodes + i] = __ldg(sph + i);
+  }
   stage_nodes(sc, snodes, n_snodes);
   uint32_t sbase = (uint32_t)__cvta_generic_to_shared(snodes);
   asm volatile("mov.u32 %0, %0;" : "+r"(sbase));  // opaque: keep it in a register instead of re-deriving it per node visit
@@ -685,7 +692,8 @@ k_extend_static(DevScene sc, DevPool pool, DevParams prm, uint32_t n_snodes) {
         float lo;
         // packed slab test and remap table in the fully staged production kernel (the counting build keeps the scalar
         // test: same decisions, and the packed one spills there)
-        const uint32_t fix = traverse<COUNT, ALL_STAGED, ALL_STAGED && !COUNT, ALL_STAGED>(sc, snodes, sbase, n_snodes, xyz(ro), xyz(rd), ro.w, RTB_TMIN, best, lo, nv, nt);
+        const uint32_t fix = traverse<COUNT, ALL_STAGED, ALL_STAGED && !COUNT, ALL_STAGED, SPHSTAGE>(
+            sc, snodes, sbase, n_snodes, xyz(ro), xyz(rd), ro.w, RTB_TMIN, best, lo, nv, nt, sbase + n_snodes * 80u);
         finish_ray(sc, pool, prm, slot, xyz(ro), xyz(rd), best);
         if (fix) queue_fix(pool, slot, fix, lo, best.hi);
       }
@@ -1447,6 +1455,10 @@ void launch_extend(const LaunchCfg& lc, const DevScene& sc, const DevPool& pool,
     if (count) {
       if (sort) k_extend_static<true, false, true><<<lc.extend_grid, RTB_EXTEND_THREADS, lc.extend_smem, st>>>(sc, pool, prm, lc.n_snodes);
       else k_extend_static<true, false, false><<<lc.extend_grid, RTB_EXTEND_THREADS, lc.extend_smem, st>>>(sc, pool, prm, lc.n_snodes);
+    } else if (lc.all_staged && lc.sphere_smem) {
+      const uint32_t smem = lc.extend_smem + lc.sphere_smem;
+      if (sort) k_extend_static<false, true, true, true><<<lc.extend_grid, RTB_EXTEND_THREADS, smem, st>>>(sc, pool, prm, lc.n_snodes);
+      else k_extend_static<false, true, false, true><<<lc.extend_grid, RTB_EXTEND_THREADS, smem, st>>>(sc, pool, prm, lc.n_snodes);
     } else if (lc.all_staged) {
       if (sort) k_extend_static<false, true, true><<<lc.extend_grid, RTB_EXTEND_THREADS, lc.extend_smem, st>>>(sc, pool, prm, lc.n_snodes);
       else k_extend_static<false, true, false><<<lc.extend_grid, RTB_EXTEND_THREADS, lc.extend_smem, st>>>(sc, pool, prm, lc.n_snodes);
@@ -1493,7 +1505,7 @@ void launch_primary_rays(const DevCameraF64& cam, uint32_t W, uint32_t H, float*
   k_primary_rays<<<cdiv(W * H, 256), 256, 0, st>>>(cam, W, H, org, dir, time);
 }
 
-int configure_launch(LaunchCfg& lc, uint32_t n_nodes, uint32_t max_depth, int sm_count) {
+int configure_launch(LaunchCfg& lc, uint32_t n_nodes, uint32_t max_depth, uint32_t n_spheres, int sm_count) {
   // stage as much of the (breadth-first ordered) node array as fits the shared-memory budget
   // extend runs 2 CTAs per SM: 2 x (stage + 2 KB list [+ 20 KB of per-warp ray/result buffers, dynamic fetch]) must fit
   // the 227 KB of an SM beside one 3 KB shade CTA
@@ -1518,6 +1530,9 @@ int configure_launch(LaunchCfg& lc, uint32_t n_nodes, uint32_t max_depth, int sm
   if (mode) lc.mode = !strcmp(mode, "static") ? EXTEND_STATIC : (!strcmp(mode, "wq") ? EXTEND_WQ : EXTEND_DYNAMIC);
   if (lc.mode == EXTEND_WQ && (lc.all_staged || max_depth + 2u > RTB_WQ_STACK))  // (pushes <= internal levels on a path)
     lc.mode = lc.dynamic_fetch ? EXTEND_DYNAMIC : EXTEND_STATIC;
+  // fully staged tree: the sphere records go to shared memory too (C1: 486 x 16 B); the leaf tests read them with LDS
+  // (only the production kernel reads them: the counting build and the other kernels launch without these bytes)
+  lc.sphere_smem = lc.mode == EXTEND_STATIC && lc.all_staged && n_spheres <= RTB_SPHERE_STAGE_BYTES / 16u ? n_spheres * 16u : 0u;
   cudaError_t e;
   const void* extend_fn = (const void*)k_extend<false>;
   if (lc.mode == EXTEND_WQ) {
@@ -1539,8 +1554,16 @@ int configure_launch(LaunchCfg& lc, uint32_t n_nodes, uint32_t max_depth, int sm
     e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)budget);
     if (e != cudaSuccess) return (int)e;
   }
+  // (only for a scene that uses them: with the attribute set on these two kernels for every scene, C4 measured 3.4 % and
+  //  C3 1.5 % slower on a B200 at 1000 W, although none of the kernels they run changed; profiles/r6_sphere_stage.md)
+  if (lc.sphere_smem) {
+    for (const void* fn : {(const void*)k_extend_static<false, true, false, true>, (const void*)k_extend_static<false, true, true, true>}) {
+      e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(budget + RTB_SPHERE_STAGE_BYTES));
+      if (e != cudaSuccess) return (int)e;
+    }
+  }
   int occ = 0;
-  e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, extend_fn, RTB_EXTEND_THREADS, lc.extend_smem);
+  e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, extend_fn, RTB_EXTEND_THREADS, lc.extend_smem + lc.sphere_smem);
   if (e != cudaSuccess) return (int)e;
   if (occ < 1) occ = 1;
   // two extend CTAs per SM (of the three that fit): leaves a third of the register file to the shade kernels of the

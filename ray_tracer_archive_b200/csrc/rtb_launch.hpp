@@ -7,6 +7,7 @@
 #define RTB_EXTEND_THREADS 256
 #endif
 #define RTB_SHADE_THREADS 256
+#define RTB_SPHERE_STAGE_BYTES (16u * 1024u)  /* shared-memory cap of the sphere records staged beside a fully staged tree */
 #ifndef RTB_SHADE_MIN_BLOCKS
 #define RTB_SHADE_MIN_BLOCKS 3
 #endif
@@ -37,12 +38,15 @@ struct LaunchCfg {
   uint32_t extend_grid = 0, shade_grid = 0, fixup_grid = 0, extend_smem = 0, n_snodes = 0;
   bool dynamic_fetch = false;
   bool all_staged = false;  // every BVH node fits the shared-memory stage: the kernel without a global node path is used
+  uint32_t sphere_smem = 0;  // > 0: ... and the sphere records (these bytes) are staged after the nodes by the production
+                             // static kernel; added to extend_smem for that kernel's launch only
   // slots that give every resident shade warp exactly one chunk: pools are sized in multiples of this
   uint32_t pool_unit = 0;
 };
 
 // max_depth: levels of the tree (the warp-queue kernel keeps fixed-depth stacks in shared memory)
-int configure_launch(LaunchCfg& lc, uint32_t n_nodes, uint32_t max_depth, int sm_count);
+// n_spheres: records of the sphere array (RTB_SPHERE_STAGE_BYTES / 16 at most are staged with a fully staged tree)
+int configure_launch(LaunchCfg& lc, uint32_t n_nodes, uint32_t max_depth, uint32_t n_spheres, int sm_count);
 int read_check_failures(unsigned int* out8);  // RTB_CHECKED build: failed bounds assertions by kind; 0xFFFFFFFF otherwise
 void launch_init_pool(const DevPool& pool, unsigned long long total_paths, cudaStream_t st);
 void launch_generate(const LaunchCfg& lc, const DevPool& pool, const DevParams& prm, const DevCamera& cam, cudaStream_t st);

@@ -7,7 +7,7 @@ reduced spp, and the two are compared.
 - Counters of an instrumented render (RTB_RENDER_COUNT): segments, node visits, primitive tests per type, exactly
   re-traced and refined rays.  They must be EQUAL: any difference means a node or primitive decision changed.
 - P1 probe (rtb_primary_rays + the production kernels): primitive ids and t BITWISE equal on every pixel.
-- bench.py --dump-outputs (C1 defaults, 1 step): counters equal; accum may differ only by the order of the float
+- bench.py --dump-outputs (C1 defaults without the C5 sub-record, 1 step): counters equal; accum may differ only by the order of the float
   atomics, bounded by the difference of two runs of the base build.
 Exit code 0 iff everything holds."""
 import argparse
@@ -57,7 +57,7 @@ def run_build(lib, out, spp_scale):
 def run_bench_dump(lib, out):
     env = dict(os.environ, RTB200_LIB=os.path.abspath(lib))
     subprocess.check_call([sys.executable, "bench.py", "--gpus", "1", "--steps", "1", "--warmup", "1", "--no-cpu-baseline",
-                           "--dump-outputs", out], env=env, cwd=ROOT, stdout=subprocess.DEVNULL)
+                           "--strong-spp", "0", "--dump-outputs", out], env=env, cwd=ROOT, stdout=subprocess.DEVNULL)
 
 
 def main():

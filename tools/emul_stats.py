@@ -37,6 +37,9 @@ for w in sys.argv[1:] or ["C3", "C4"]:
         n = len(o32)
         print(f"{w} bounce {bounce}: {n} rays, {s[0] / n:.2f} node visits/ray, {s[1] / max(s[0], 1):.3f} of them without a hit child, "
               f"{s[2] / n:.2f} internal + {s[3] / n:.2f} leaf children hit/ray, {nt / n:.2f} prim tests/ray")
+        nl = max(s[4] + s[5] + s[6], 1)
+        print(f"      visits with leaf hits: {(s[4] + s[5] + s[6]) / n:.2f}/ray, holding 1 / 2 / 3+ primitives: "
+              f"{s[4] / nl:.3f} / {s[5] / nl:.3f} / {s[6] / nl:.3f}, {s[7] / nl:.2f} primitives per such visit")
         # the same rays again with t_max initialised to the hit distance found: what perfect culling of stale stack entries
         # (groups pushed before the hit was known) could save at most
         t0 = np.where(ids != H.NONE, ts * (1 + 3e-4), np.inf).astype(np.float32)
