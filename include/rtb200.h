@@ -293,6 +293,33 @@ int rtb_render(rtb_context* ctx, rtb_scene* scene, const rtb_camera* cam, const 
  * the host only up to the internal termination checks; on return the work is complete on `stream`. */
 int rtb_render_device(rtb_context* ctx, rtb_scene* scene, const rtb_camera* cam, const rtb_params* params,
                       void* d_accum, void* stream, rtb_stats* stats);
+/* ---- denoiser guide buffers (AOVs, "arbitrary output variables") ------------------------------------------------------
+ * Albedo, normal and depth images of the same sample set a render with the same rtb_params draws: global sample indices
+ * [sample_offset, sample_offset + spp) of every pixel.  Sample s of pixel p traces exactly the FIRST ray of that render
+ * sample (the same jitter, thin-lens and shutter-time draws), and its closest hit comes from the render's own extend
+ * kernels, including the exact f64 pass.  A ConstantMedium decides its scatter distance from the path's own stream at
+ * segment 1, as in the render.  Denoisers (OIDN, the OptiX denoiser) take these as guides of a low-spp render.
+ *
+ * Output: 8 floats per pixel, (H, W, 8) float32, row 0 = top.  Each value is a SUM over samples, like the accumulation
+ * buffer, so calls compose with sample_offset, RTB_RENDER_ACCUMULATE and a caller's own reduce across ranks:
+ *   [0..2] albedo, each channel clamped to [0, 1]:
+ *            Lambertian, Metal, Isotropic: the texture value at the hit (the attenuation the integrator applies);
+ *            Dielectric: (1, 1, 1); DiffuseLight: the emitted colour on its front face, else 0; a miss: params->background
+ *   [3]    coverage: 1 if the ray hit a surface or scattered in a medium, else 0
+ *   [4..6] shading normal: world space, unit length, facing the ray (the normal the integrator scatters about, including
+ *          RotateY's front_face rule, hittable.rs:173); (0, 0, 0) for a medium scatter or a miss
+ *   [7]    depth: t * |d|, the distance from the ray origin (the lens point) to the hit or scatter point; 0 for a miss
+ * Divide albedo, coverage and normal by spp and depth by the coverage sum.  A sample with a non-finite value is skipped
+ * and counted in stats->rejected.  stats->paths = stats->segments = W * H * spp.
+ * Arguments are checked as by rtb_render_device; the only accepted flag is RTB_RENDER_ACCUMULATE.  A multi-device context
+ * returns RTB_ERR_UNSUPPORTED: split the samples over per-device contexts with sample_offset and sum the buffers.
+ * rtb_render_aov_device: d_aov is a DEVICE pointer to W*H*8 floats, stream a cudaStream_t (NULL = default stream); on
+ * return the work is complete on `stream`.
+ * rtb_render_aov: into the context's own buffer; if aov_out != NULL copies W*H*8 floats back to the host. */
+int rtb_render_aov_device(rtb_context* ctx, rtb_scene* scene, const rtb_camera* cam, const rtb_params* params, void* d_aov,
+                          void* stream, rtb_stats* stats);
+int rtb_render_aov(rtb_context* ctx, rtb_scene* scene, const rtb_camera* cam, const rtb_params* params, float* aov_out,
+                   rtb_stats* stats);
 /* write_color (main.rs:141-169): /total_spp, NaN->0, sqrt, clamp [0,0.999], *256 -> u8.  d_accum device, rgb8_out host. */
 int rtb_finalize_rgb8(rtb_context* ctx, const void* d_accum, uint32_t width, uint32_t height, uint32_t total_spp,
                       uint8_t* rgb8_out);

@@ -150,6 +150,12 @@ extern "C" {
                       stats: *mut RtbStats) -> c_int;
     pub fn rtb_render_device(ctx: *mut RtbContext, s: *mut RtbScene, cam: *const RtbCamera, p: *const RtbParams,
                              d_accum: *mut c_void, stream: *mut c_void, stats: *mut RtbStats) -> c_int;
+    // denoiser guide buffers (W*H*8 float sums: albedo rgb, coverage, normal xyz, depth; see rtb200.h).  Declared for
+    // callers of the shim; this file is not compiled in the project's own build and test image.
+    pub fn rtb_render_aov_device(ctx: *mut RtbContext, s: *mut RtbScene, cam: *const RtbCamera, p: *const RtbParams,
+                                 d_aov: *mut c_void, stream: *mut c_void, stats: *mut RtbStats) -> c_int;
+    pub fn rtb_render_aov(ctx: *mut RtbContext, s: *mut RtbScene, cam: *const RtbCamera, p: *const RtbParams,
+                          aov_out: *mut f32, stats: *mut RtbStats) -> c_int;
     pub fn rtb_finalize_rgb8(ctx: *mut RtbContext, d_accum: *const c_void, w: u32, h: u32, total_spp: u32, out: *mut u8) -> c_int;
     pub fn rtb_primary_hits(ctx: *mut RtbContext, s: *mut RtbScene, cam: *const RtbCamera, w: u32, h: u32, prim_id: *mut u32,
                             t: *mut f32, stats: *mut RtbStats) -> c_int;

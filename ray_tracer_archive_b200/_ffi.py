@@ -123,6 +123,8 @@ SIGNATURES = {
     "rtb_scene_export_exact": (_I, [_VP, _U32, _VP, _SZ, C.POINTER(C.c_float), C.POINTER(C.c_float)]),
     "rtb_render": (_I, [_VP, _VP, C.POINTER(Camera), C.POINTER(Params), _VP, C.POINTER(Stats)]),
     "rtb_render_device": (_I, [_VP, _VP, C.POINTER(Camera), C.POINTER(Params), _VP, _VP, C.POINTER(Stats)]),
+    "rtb_render_aov": (_I, [_VP, _VP, C.POINTER(Camera), C.POINTER(Params), _VP, C.POINTER(Stats)]),
+    "rtb_render_aov_device": (_I, [_VP, _VP, C.POINTER(Camera), C.POINTER(Params), _VP, _VP, C.POINTER(Stats)]),
     "rtb_finalize_rgb8": (_I, [_VP, _VP, _U32, _U32, _U32, _VP]),
     "rtb_primary_hits": (_I, [_VP, _VP, C.POINTER(Camera), _U32, _U32, _VP, _VP, C.POINTER(Stats)]),
     "rtb_trace_rays": (_I, [_VP, _VP, _VP, _VP, _VP, _U32, _VP, _VP, C.POINTER(Stats)]),

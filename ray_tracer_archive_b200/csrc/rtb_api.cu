@@ -76,6 +76,7 @@ struct rtb_context {
   DevCounters* h_counters = nullptr;   // pinned
   // image-sized buffers
   DevBuf<float4> accum;
+  DevBuf<float4> aov;  // rtb_render_aov's sums, 2 per pixel (kept apart from accum: either call may accumulate)
   DevBuf<uint32_t> pix_order;
   uint32_t pix_w = 0, pix_h = 0;
   DevBuf<uint8_t> rgb8;
@@ -901,36 +902,67 @@ static int ensure_pix_order(rtb_context* c, uint32_t W, uint32_t H, cudaStream_t
   return RTB_OK;
 }
 
-int rtb_render_device(rtb_context* c, rtb_scene* s, const rtb_camera* cam, const rtb_params* p, void* d_accum,
-                      void* stream, rtb_stats* stats) {
-  if (!c || !s || !cam || !p || !d_accum) return set_err(RTB_ERR_INVALID, "NULL argument");
+#define RTB_DEFAULT_POOL (1u << 22)  // path-pool slots of all lanes together when rtb_params::pool_paths is 0
+
+// the argument checks rtb_render_device and rtb_render_aov_device share
+static int check_render_args(rtb_context* c, rtb_scene* s, const rtb_camera* cam, const rtb_params* p, const void* buf) {
+  if (!c || !s || !cam || !p || !buf) return set_err(RTB_ERR_INVALID, "NULL argument");
   if (!s->committed) return set_err(RTB_ERR_STATE, "scene not committed (call rtb_scene_commit)");
   if (p->width < 2 || p->height < 2) return set_err(RTB_ERR_INVALID, "image must be at least 2x2 (u = (i+xi)/(W-1), main.rs:752)");
   if (p->max_depth < 1 || p->max_depth > 255) return set_err(RTB_ERR_INVALID, "max_depth must be in [1,255]");
   if (p->spp == 0) return set_err(RTB_ERR_INVALID, "spp must be > 0");
   if ((uint64_t)p->sample_offset + p->spp > (1u << 24)) return set_err(RTB_ERR_INVALID, "sample index exceeds 2^24");
-  CU(cudaSetDevice(c->device));
-  cudaStream_t st = (cudaStream_t)stream;
-  const uint64_t npix = (uint64_t)p->width * p->height;
-  const bool count = (p->flags & RTB_RENDER_COUNT) != 0, time_ext = (p->flags & RTB_RENDER_TIME_EXTEND) != 0;
-  // lanes: concurrent wavefront instances on disjoint sample ranges (instrumented runs use one lane so that the
-  // per-launch timings / counters describe the kernel alone)
-  // 4 lanes: C1 7696 -> 7882, C3 +2.6 % against 3; the dynamic-fetch kernel at 64 registers co-schedules the extend CTAs of
-  // four lanes on an SM: C4 3915 (3 lanes) -> 4096 (4), 5 / 6 lanes add nothing (profiles/r3_ab.md §9)
-  static const int env_lanes = getenv("RTB_LANES") ? atoi(getenv("RTB_LANES")) : 0;
-  const int want_lanes = env_lanes > 0 ? env_lanes : 4;
-  int n_lanes = (count || time_ext) ? 1 : std::max(1, std::min(want_lanes, RTB_MAX_LANES));
-  if ((uint32_t)n_lanes > p->spp) n_lanes = (int)p->spp;
-  uint32_t pool_total = p->pool_paths ? p->pool_paths : (1u << 22);  // all lanes together; 112 B per slot
-  int rc = ensure_pix_order(c, p->width, p->height, st);
-  if (rc) return rc;
-  DevCamera dcam;
+  return RTB_OK;
+}
+
+// the f32 camera of the render's primary rays; refuses a camera whose basis is not finite
+static int render_camera(const rtb_camera& cam, DevCamera& dcam) {
   DevCameraF64 dcam64;
-  camera_basis(*cam, dcam, dcam64);
+  camera_basis(cam, dcam, dcam64);
   for (int a = 0; a < 3; ++a)  // lookfrom == lookat, vup parallel to the view direction, NaN / inf arguments
     if (!std::isfinite(dcam.origin[a]) || !std::isfinite(dcam.lmo[a]) || !std::isfinite(dcam.horizontal[a]) || !std::isfinite(dcam.vertical[a]) ||
         !std::isfinite(dcam.u[a]) || !std::isfinite(dcam.v[a]))
       return set_err(RTB_ERR_INVALID, "degenerate camera (non-finite basis: lookfrom == lookat, vup along the view direction, or non-finite arguments)");
+  return RTB_OK;
+}
+
+// DevParams::opt of the scene's extend launches.  Per-scene scheduling of the extend kernel (profiles/r3_ab.md): deep trees
+// (dynamic fetch) park their leaf tests, trees that do not fit the shared-memory stage order each chunk's rays by direction
+// octant, small staged trees do neither.  RTB_OPT overrides (experiments).
+static uint32_t extend_opt(const rtb_scene* s) {
+  static const char* env_opt = getenv("RTB_OPT");
+  return env_opt ? (uint32_t)atoi(env_opt)
+         : s->lc.mode == EXTEND_WQ ? ((24u << RTB_OPT_PARK_SHIFT) | (2u << 16))  // serve queues of >= 24 rays, 2 tests per ray and round
+         : s->lc.mode == EXTEND_DYNAMIC ? (14u << RTB_OPT_PARK_SHIFT)
+                                        : (s->lc.all_staged ? 0u : 2u /* RTB_OPT_OCTANT_SORT */);
+}
+
+// lanes: concurrent wavefront instances on disjoint sample ranges
+// 4 lanes: C1 7696 -> 7882, C3 +2.6 % against 3; the dynamic-fetch kernel at 64 registers co-schedules the extend CTAs of
+// four lanes on an SM: C4 3915 (3 lanes) -> 4096 (4), 5 / 6 lanes add nothing (profiles/r3_ab.md §9)
+static int default_lanes() {
+  static const int env_lanes = getenv("RTB_LANES") ? atoi(getenv("RTB_LANES")) : 0;
+  const int want_lanes = env_lanes > 0 ? env_lanes : 4;
+  return std::max(1, std::min(want_lanes, RTB_MAX_LANES));
+}
+
+int rtb_render_device(rtb_context* c, rtb_scene* s, const rtb_camera* cam, const rtb_params* p, void* d_accum,
+                      void* stream, rtb_stats* stats) {
+  int rc = check_render_args(c, s, cam, p, d_accum);
+  if (rc) return rc;
+  CU(cudaSetDevice(c->device));
+  cudaStream_t st = (cudaStream_t)stream;
+  const uint64_t npix = (uint64_t)p->width * p->height;
+  const bool count = (p->flags & RTB_RENDER_COUNT) != 0, time_ext = (p->flags & RTB_RENDER_TIME_EXTEND) != 0;
+  // instrumented runs use one lane so that the per-launch timings / counters describe the kernel alone
+  int n_lanes = (count || time_ext) ? 1 : default_lanes();
+  if ((uint32_t)n_lanes > p->spp) n_lanes = (int)p->spp;
+  uint32_t pool_total = p->pool_paths ? p->pool_paths : RTB_DEFAULT_POOL;  // all lanes together; 112 B per slot
+  rc = ensure_pix_order(c, p->width, p->height, st);
+  if (rc) return rc;
+  DevCamera dcam;
+  rc = render_camera(*cam, dcam);
+  if (rc) return rc;
 
   struct LaneRun { DevPool pool; DevParams prm; unsigned long long total; bool active; uint64_t iters, iter_cap; };
   LaneRun run[RTB_MAX_LANES];
@@ -955,14 +987,7 @@ int rtb_render_device(rtb_context* c, rtb_scene* s, const rtb_camera* cam, const
     for (int a = 0; a < 3; ++a) prm.bg[a] = p->background[a];
     prm.pix_order = c->pix_order.p;
     prm.inv_npix = 1.0 / (double)npix;
-    static const char* env_opt = getenv("RTB_OPT");
-    // per-scene scheduling of the extend kernel (profiles/r3_ab.md): deep trees (dynamic fetch) park their leaf tests,
-    // trees that do not fit the shared-memory stage order each chunk's rays by direction octant, small staged trees do
-    // neither.  RTB_OPT overrides (experiments).
-    prm.opt = env_opt ? (uint32_t)atoi(env_opt)
-              : s->lc.mode == EXTEND_WQ ? ((24u << RTB_OPT_PARK_SHIFT) | (2u << 16))  // serve queues of >= 24 rays, 2 tests per ray and round
-              : s->lc.mode == EXTEND_DYNAMIC ? (14u << RTB_OPT_PARK_SHIFT)
-                                             : (s->lc.all_staged ? 0u : 2u /* RTB_OPT_OCTANT_SORT */);
+    prm.opt = extend_opt(s);
     prm.inv_wm1 = (float)(1.0 / (double)(p->width - 1));
     prm.inv_hm1 = (float)(1.0 / (double)(p->height - 1));
     prm.accum = (float4*)d_accum;
@@ -1213,6 +1238,119 @@ int rtb_render(rtb_context* c, rtb_scene* s, const rtb_camera* cam, const rtb_pa
   int rc = rtb_render_device(c, s, cam, p, c->accum.p, nullptr, stats);
   if (rc) return rc;
   if (accum_out) CU(cudaMemcpy(accum_out, c->accum.p, npix * sizeof(float4), cudaMemcpyDeviceToHost));
+  return RTB_OK;
+}
+
+// ---- denoiser guide buffers ---------------------------------------------------------------------------------------------
+// The first segment of every sample a render with the same params traces, through the production extend + k_fixup.  The
+// W*H*spp paths are numbered as the render numbers them (start_path) and processed in batches of one lane pool each; batch
+// b runs on lane b % n_lanes, so one lane's fill / collect overlaps another lane's extend.  A lane's pool is initialised
+// once: k_fixup leaves the per-launch counters cleared, so the lane's totals (exact rays, rejected samples) add up over its
+// batches.
+int rtb_render_aov_device(rtb_context* c, rtb_scene* s, const rtb_camera* cam, const rtb_params* p, void* d_aov,
+                          void* stream, rtb_stats* stats) {
+  int rc = check_render_args(c, s, cam, p, d_aov);
+  if (rc) return rc;
+  if (p->flags & ~RTB_RENDER_ACCUMULATE) return set_err(RTB_ERR_INVALID, "rtb_render_aov accepts no flag but RTB_RENDER_ACCUMULATE");
+  if (!c->peers.empty())
+    return set_err(RTB_ERR_UNSUPPORTED, "rtb_render_aov runs on one device: split the samples with sample_offset and sum the buffers");
+  CU(cudaSetDevice(c->device));
+  cudaStream_t st = (cudaStream_t)stream;
+  const uint64_t npix = (uint64_t)p->width * p->height, total = npix * p->spp;
+  rc = ensure_pix_order(c, p->width, p->height, st);
+  if (rc) return rc;
+  DevCamera dcam;
+  rc = render_camera(*cam, dcam);
+  if (rc) return rc;
+  DevParams prm;
+  std::memset(&prm, 0, sizeof(prm));
+  prm.width = p->width; prm.height = p->height; prm.spp = p->spp; prm.sample_offset = p->sample_offset;
+  prm.max_depth = p->max_depth; prm.rr_start = p->rr_start_depth; prm.seed = p->seed;
+  for (int a = 0; a < 3; ++a) prm.bg[a] = p->background[a];
+  prm.pix_order = c->pix_order.p;
+  prm.inv_npix = 1.0 / (double)npix;
+  prm.opt = extend_opt(s);
+  prm.inv_wm1 = (float)(1.0 / (double)(p->width - 1));
+  prm.inv_hm1 = (float)(1.0 / (double)(p->height - 1));
+
+  // one round of batches = the pool of all lanes together (pool_paths, as for the render), split as evenly as it goes
+  const uint64_t round = std::min<uint64_t>(p->pool_paths ? p->pool_paths : RTB_DEFAULT_POOL, total);
+  const int n_lanes = (int)std::min<uint64_t>((uint64_t)default_lanes(), round);
+  DevPool pool[RTB_MAX_LANES];
+  for (int k = 0; k < n_lanes; ++k) {
+    const uint32_t n = (uint32_t)(round / n_lanes + ((uint64_t)k < round % n_lanes ? 1u : 0u));
+    rc = ensure_pool(c->lanes[k], n);
+    if (rc) return rc;
+    pool[k] = lane_pool(c->lanes[k], n);
+  }
+  float4* aov = (float4*)d_aov;
+  uint64_t launches = 0, extend_launches = 0;
+  CU(cudaEventRecord(c->ev0, st));
+  if (!(p->flags & RTB_RENDER_ACCUMULATE)) CU(cudaMemsetAsync(d_aov, 0, npix * 2 * sizeof(float4), st));
+  CU(cudaEventRecord(c->ev_fork, st));
+  for (int k = 0; k < n_lanes; ++k) {
+    CU(cudaStreamWaitEvent(c->lanes[k].stream, c->ev_fork, 0));
+    launch_init_pool(pool[k], 0ull, c->lanes[k].stream);
+    launches += 1;
+  }
+  for (uint64_t first = 0, b = 0; first < total; ++b) {
+    const int k = (int)(b % (uint64_t)n_lanes);
+    const cudaStream_t ls = c->lanes[k].stream;
+    const uint32_t n = (uint32_t)std::min<uint64_t>(pool[k].n, total - first);
+    launch_aov_fill(pool[k], prm, dcam, first, n, ls);
+    launch_extend(s->lc, s->dev, pool[k], prm, false, ls);
+    launch_fixup(s->lc, s->dev, pool[k], prm, ls);
+    launch_aov_collect(s->dev, pool[k], prm, aov, n, ls);
+    launches += 4;
+    extend_launches += 1;
+    first += n;
+  }
+  cudaError_t e = cudaGetLastError();
+  for (int k = 0; k < n_lanes && e == cudaSuccess; ++k) {
+    Lane& L = c->lanes[k];
+    e = cudaMemcpyAsync(L.h_counters, L.counters.p, sizeof(DevCounters), cudaMemcpyDeviceToHost, L.stream);
+    if (e == cudaSuccess) e = cudaEventRecord(L.done, L.stream);
+    if (e == cudaSuccess) e = cudaStreamWaitEvent(st, L.done, 0);
+  }
+  if (e != cudaSuccess) {  // nothing may still be writing the caller's buffer
+    for (int k = 0; k < n_lanes; ++k) cudaStreamSynchronize(c->lanes[k].stream);
+    return set_err(RTB_ERR_CUDA, std::string("aov pass: ") + cudaGetErrorString(e));
+  }
+  CU(cudaEventRecord(c->ev1, st));
+  CU(cudaEventSynchronize(c->ev1));
+  CU(cudaGetLastError());
+  if (stats) {
+    std::memset(stats, 0, sizeof(*stats));
+    float ms = 0;
+    cudaEventElapsedTime(&ms, c->ev0, c->ev1);
+    stats->paths = total;
+    stats->segments = total;
+    for (int k = 0; k < n_lanes; ++k) {
+      const DevCounters* h = c->lanes[k].h_counters;
+      stats->rejected += h->rejected;
+      stats->exact_rays += h->redone - h->refined;
+      stats->refined_rays += h->refined;
+    }
+    stats->launches = launches;
+    stats->extend_launches = extend_launches;
+    stats->ms_total = ms;
+    stats->ms_render = ms;
+    stats->n_devices = 1;
+  }
+  return RTB_OK;
+}
+
+int rtb_render_aov(rtb_context* c, rtb_scene* s, const rtb_camera* cam, const rtb_params* p, float* aov_out,
+                   rtb_stats* stats) {
+  if (!c || !p) return set_err(RTB_ERR_INVALID, "NULL argument");
+  if (!c->peers.empty())
+    return set_err(RTB_ERR_UNSUPPORTED, "rtb_render_aov runs on one device: split the samples with sample_offset and sum the buffers");
+  CU(cudaSetDevice(c->device));
+  const size_t npix = (size_t)p->width * p->height;
+  CU(c->aov.resize(npix * 2));
+  int rc = rtb_render_aov_device(c, s, cam, p, c->aov.p, nullptr, stats);
+  if (rc) return rc;
+  if (aov_out) CU(cudaMemcpy(aov_out, c->aov.p, npix * 2 * sizeof(float4), cudaMemcpyDeviceToHost));
   return RTB_OK;
 }
 

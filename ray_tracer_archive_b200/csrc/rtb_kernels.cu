@@ -1295,6 +1295,51 @@ __global__ void k_probe_collect(DevScene sc, DevPool pool, uint32_t n, uint32_t*
   t_out[i] = h.x;
 }
 
+// ---- denoiser guide buffers (rtb_render_aov): the first segment of every render sample, traced by the production extend +
+// k_fixup over a pool these two kernels fill and read ---------------------------------------------------------------------
+// slot i holds path number first_path + i: start_path() is the render's own path start, so the ray is that sample's first ray
+__global__ void k_aov_fill(DevPool pool, DevParams prm, DevCamera cam, unsigned long long first_path, uint32_t n) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= pool.n_chunks * RTB_CHUNK) return;
+  if (i < n) {
+    start_path(pool, prm, cam, i, first_path + i);
+    if (!(prm.opt & RTB_OPT_OCTANT_SORT)) pool.cls[i] = (uint8_t)CLS_NEW;
+  } else {
+    pool.cls[i] = (uint8_t)CLS_DEAD;
+  }
+}
+
+// per-sample (albedo, coverage) and (shading normal, depth) of the hit record, summed into aov[2 pixel], aov[2 pixel + 1]
+__global__ void __launch_bounds__(RTB_SHADE_THREADS) k_aov_collect(DevScene sc, DevPool pool, DevParams prm, float4* aov,
+                                                                  uint32_t n) {
+  const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const float4 h = pool.hit[i];
+  const uint32_t pixel = __float_as_uint(pool.st[2 * i].w), ref = __float_as_uint(h.y);
+  float3 albedo = f3(prm.bg[0], prm.bg[1], prm.bg[2]), n3 = f3(0.f, 0.f, 0.f);
+  float cover = 0.f, depth = 0.f;
+  if (ref != REF_MISS) {
+    const float4 ro = pool.ray[2 * i], rd = pool.ray[2 * i + 1];
+    const Surf s = surface_at(sc, ref, __float_as_uint(h.z), xyz(ro), xyz(rd), ro.w, h.x);
+    const float4 m = __ldg(&sc.materials[2 * s.mat]);
+    const uint32_t type = __float_as_uint(m.x);
+    if (type == RTB_MAT_DIELECTRIC) albedo = f3(1.f, 1.f, 1.f);
+    else if (type == RTB_MAT_DIFFUSE_LIGHT && !s.front) albedo = f3(0.f, 0.f, 0.f);
+    else albedo = tex_value(sc, m, s.mat, s);
+    if ((ref >> REF_TYPE_SHIFT) != PT_MEDIUM) n3 = s.n;
+    cover = 1.f;
+    depth = h.x * sqrtf(dot(xyz(rd), xyz(rd)));
+  }
+  if (!(isfinite(albedo.x) && isfinite(albedo.y) && isfinite(albedo.z) && isfinite(n3.x) && isfinite(n3.y) &&
+        isfinite(n3.z) && isfinite(depth))) {  // deposit()'s policy: a non-finite sample is dropped and counted
+    atomicAdd(&pool.c->rejected, 1ull);
+    return;
+  }
+  albedo = f3(__saturatef(albedo.x), __saturatef(albedo.y), __saturatef(albedo.z));
+  red_add_v4(aov + 2 * (size_t)pixel, albedo.x, albedo.y, albedo.z, cover);
+  red_add_v4(aov + 2 * (size_t)pixel + 1, n3.x, n3.y, n3.z, depth);
+}
+
 // pixel-centre primary rays, generated in f64 like the reference's camera (camera.rs:60-70) and rounded once
 __global__ void k_primary_rays(DevCameraF64 cam, uint32_t W, uint32_t H, float* __restrict__ org, float* __restrict__ dir,
                                float* __restrict__ time) {
@@ -1499,6 +1544,14 @@ void launch_bw_global(const uint4* p, size_t n_vec, uint32_t reps, uint4* sink, 
 }
 void launch_bw_shared(uint32_t reps, uint4* sink, uint32_t grid, cudaStream_t st) {
   k_bw_shared<<<grid, 256, 32768, st>>>(reps, sink);
+}
+void launch_aov_fill(const DevPool& pool, const DevParams& prm, const DevCamera& cam, unsigned long long first_path,
+                     uint32_t n, cudaStream_t st) {
+  k_aov_fill<<<cdiv(pool.n_chunks * RTB_CHUNK, 256), 256, 0, st>>>(pool, prm, cam, first_path, n);
+}
+void launch_aov_collect(const DevScene& sc, const DevPool& pool, const DevParams& prm, float4* aov, uint32_t n,
+                        cudaStream_t st) {
+  k_aov_collect<<<cdiv(n, RTB_SHADE_THREADS), RTB_SHADE_THREADS, 0, st>>>(sc, pool, prm, aov, n);
 }
 void launch_primary_rays(const DevCameraF64& cam, uint32_t W, uint32_t H, float* org, float* dir, float* time,
                          cudaStream_t st) {

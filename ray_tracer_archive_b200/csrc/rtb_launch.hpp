@@ -59,6 +59,12 @@ void launch_shade(const LaunchCfg& lc, const DevScene& sc, const DevPool& pool, 
 void launch_finalize(const float4* accum, uint8_t* rgb, uint32_t npix, float inv_spp, cudaStream_t st);
 void launch_probe_fill(const DevPool& pool, const float* org, const float* dir, const float* time, uint32_t n, cudaStream_t st);
 void launch_probe_collect(const DevScene& sc, const DevPool& pool, uint32_t n, uint32_t* id_out, float* t_out, cudaStream_t st);
+// denoiser guide buffers: slot i of `pool` starts path number first_path + i (i < n); the hit records of those slots are
+// then summed as 8 floats per pixel into aov (2 float4 per pixel)
+void launch_aov_fill(const DevPool& pool, const DevParams& prm, const DevCamera& cam, unsigned long long first_path,
+                     uint32_t n, cudaStream_t st);
+void launch_aov_collect(const DevScene& sc, const DevPool& pool, const DevParams& prm, float4* aov, uint32_t n,
+                        cudaStream_t st);
 void launch_primary_rays(const DevCameraF64& cam, uint32_t W, uint32_t H, float* org, float* dir, float* time,
                          cudaStream_t st);
 void launch_bw_global(const uint4* p, size_t n_vec, uint32_t reps, uint4* sink, uint32_t grid, cudaStream_t st);

@@ -46,6 +46,36 @@ def save_image(path: str, rgb8: np.ndarray) -> None:
     Image.fromarray(a).save(path, quality=100)
 
 
+# ---- denoiser guide images (rtb_render_aov) ----------------------------------------------------------------------------
+def aov_images(sums: np.ndarray, spp: int) -> dict:
+    """(H, W, 8) sums of rtb_render_aov over `spp` samples -> {"albedo" (H,W,3), "normal" (H,W,3), "depth" (H,W),
+    "coverage" (H,W)} float32.  Albedo, normal and coverage are means over the samples; depth is the mean over the samples
+    that hit something (0 where none did).  The normal is the mean of unit vectors, so it is shorter than 1 at edges."""
+    a = np.asarray(sums, dtype=np.float32)
+    if a.ndim != 3 or a.shape[2] != 8:
+        raise ValueError("AOV sums must have shape (H, W, 8)")
+    if spp <= 0:
+        raise ValueError("spp must be > 0")
+    inv = np.float32(1.0 / spp)
+    cover = a[..., 3]
+    depth = np.zeros_like(cover)
+    np.divide(a[..., 7], cover, out=depth, where=cover > 0)
+    return {"albedo": a[..., 0:3] * inv, "normal": a[..., 4:7] * inv, "depth": depth, "coverage": cover * inv}
+
+
+def save_pfm(path: str, img: np.ndarray) -> None:
+    """Portable float map: (H, W) -> "Pf", (H, W, 3) -> "PF"; row 0 = top as everywhere here.  Written little-endian
+    (negative scale) with rows bottom-up, as the format stores them; OIDN's example tool reads it."""
+    a = np.asarray(img, dtype=np.float32)
+    if a.ndim == 3 and a.shape[2] == 1:
+        a = a[..., 0]
+    if not (a.ndim == 2 or (a.ndim == 3 and a.shape[2] == 3)):
+        raise ValueError("PFM takes (H, W) or (H, W, 3) images")
+    with open(path, "wb") as f:
+        f.write(b"%s\n%d %d\n-1.0\n" % (b"Pf" if a.ndim == 2 else b"PF", a.shape[1], a.shape[0]))
+        f.write(np.ascontiguousarray(a[::-1], dtype="<f4").tobytes())
+
+
 # ---- checkpoint / resume of the accumulation buffer (SURVEY §8f row 3: "resume = add more spp") -----------------------
 # The accumulation buffer holds SUMS over samples (main.rs:767-781) and samples are keyed by their global index, so a
 # render can be continued later — or on another GPU — by loading the sums, passing sample_offset = samples already

@@ -203,6 +203,21 @@ class Scene:
                                            C.c_void_p(stream_ptr), C.byref(st)))
         return st.as_dict()
 
+    def render_aov(self, cam: F.Camera, params: F.Params, readback: bool = True):
+        """rtb_render_aov: denoiser guide sums of the render's first segments -> ((H,W,8) float32 or None, stats dict).
+        Per pixel: albedo rgb, coverage, shading normal xyz, depth, each summed over samples (io.aov_images divides)."""
+        st = F.Stats()
+        out = np.empty((params.height, params.width, 8), dtype=np.float32) if readback else None
+        F.check(self.lib.rtb_render_aov(self.ctx.h, self.h, C.byref(cam), C.byref(params), F.ptr(out), C.byref(st)))
+        return out, st.as_dict()
+
+    def render_aov_device(self, cam: F.Camera, params: F.Params, d_ptr: int, stream_ptr: int = 0):
+        """rtb_render_aov_device: sum the guide values into a caller-owned device buffer of W*H*8 floats."""
+        st = F.Stats()
+        F.check(self.lib.rtb_render_aov_device(self.ctx.h, self.h, C.byref(cam), C.byref(params), C.c_void_p(d_ptr),
+                                               C.c_void_p(stream_ptr), C.byref(st)))
+        return st.as_dict()
+
     def finalize_rgb8(self, width, height, total_spp, d_accum_ptr: int = 0):
         out = np.empty((height, width, 3), dtype=np.uint8)
         F.check(self.lib.rtb_finalize_rgb8(self.ctx.h, C.c_void_p(d_accum_ptr) if d_accum_ptr else None, width, height,
