@@ -219,6 +219,24 @@ int rtb_scene_set_perlin(rtb_scene* s, uint32_t table_id, const double* ranvec_2
                          const uint32_t* perm_y, const uint32_t* perm_z);
 int rtb_scene_set_mesh(rtb_scene* s, uint32_t mesh_id, const float* vertices_xyz, uint32_t n_vertices,
                        const uint32_t* indices, uint32_t n_triangles);
+/* Smooth shading and texture coordinates of a mesh set with rtb_scene_set_mesh (call it after that call; a later
+ * rtb_scene_set_mesh of the same id clears them).  Like the mesh itself, the attributes are read when the graph is
+ * flattened: call both before rtb_scene_set_graph, and set the graph again (then commit) to change them later.
+ * Each stream has its own index stream, as in OBJ: normal_indices / uv_indices hold n_triangles x 3 indices into the
+ * stream's own array, or are NULL to reuse the mesh's position indices (then the count must equal the vertex count).
+ * normals_xyz = NULL: no vertex normals; uvs_2 = NULL: no texture coordinates.  Normals are normalised on the host in f64
+ * and rounded to f32; a zero normal is accepted.  Out-of-range indices, count mismatches and non-finite values are
+ * RTB_ERR_INVALID.  Geometry is untouched: hits, t and primitive ids are the same with and without attributes.
+ * Shading, with (b1, b2) the hit's barycentrics and b0 = 1 - b1 - b2:
+ *   ns = normalize(b0 n0 + b1 n1 + b2 n2) in world space (the RotateY of the wrapper chain turns the normals, Translate
+ *   does not), flipped to the side of the ray-facing geometric normal; the geometric normal when that sum is non-finite
+ *   or shorter than 1e-10.  front_face and the FlipFace / RotateY face rules stay on the geometric normal; ns replaces
+ *   the normal in scattering and in the AOV normal channel.  No normal bending: a scattered ray that points below the
+ *   geometric surface is traced as it is.
+ *   (u, v) = b0 uv0 + b1 uv1 + b2 uv2 replaces the barycentrics as texture coordinates (ImageTexture clamps to [0, 1]). */
+int rtb_scene_set_mesh_attributes(rtb_scene* s, uint32_t mesh_id, const float* normals_xyz, uint32_t n_normals,
+                                  const uint32_t* normal_indices, const float* uvs_2, uint32_t n_uvs,
+                                  const uint32_t* uv_indices);
 int rtb_scene_set_lights(rtb_scene* s, const rtb_light* lights, uint32_t n);
 /* Limits (RTB_ERR_UNSUPPORTED beyond them): at most 8 entries in the light list and 8 ConstantMedium objects per scene (both
  * live in the kernels' constant bank: every shaded hit walks the light list, every ray tests every medium boundary; the
@@ -281,6 +299,11 @@ int rtb_scene_export_prims(rtb_scene* s, uint32_t type /*0 sphere 1 moving 2 qua
  * two rounding scales of the f32 quad test.  Any pointer may be NULL. */
 int rtb_scene_export_exact(rtb_scene* s, uint32_t type, double* records, size_t cap_bytes, float* coord_max,
                            float* eps_ab);
+/* leaf-ordered shading records of the triangles (the order of rtb_scene_export_prims(type 3)), 16 floats = 64 bytes each:
+ *   [0..2] n0  [3] u0  [4..6] n1  [7] u1  [8..10] n2  [11] u2  [12] v0  [13] v1  [14] v2  [15] flags (uint32 bits)
+ * with world-space unit vertex normals n0..n2, texture coordinates (u_k, v_k) and flags bit 0 = normals, bit 1 = uvs.
+ * A triangle without attributes has an all-zero record.  cap_bytes must hold 64 x the triangle count. */
+int rtb_scene_export_triangle_attributes(rtb_scene* s, float* records, size_t cap_bytes);
 
 /* ---- the hot path ------------------------------------------------------------------------------------------ */
 /* Renders params->spp samples of every pixel into the context's float4 accumulation buffer

@@ -132,6 +132,10 @@ struct BVHNode : Hittable {                                             // bvh.r
 };
 struct TriangleMesh : Hittable {                                        // new (SURVEY §8a N1): OBJ-style indexed mesh
   std::vector<float> vertices; std::vector<uint32_t> indices; MaterialPtr mat_ptr;
+  // optional smooth shading / texture coordinates (rtb_scene_set_mesh_attributes): xyz per normal, uv per texture
+  // coordinate, each with its own per-corner indices (empty: the position indices)
+  std::vector<float> normals; std::vector<uint32_t> normal_indices;
+  std::vector<float> uvs; std::vector<uint32_t> uv_indices;
 };
 
 // ------------------------------------------------------------------------------------------------ records
@@ -221,6 +225,13 @@ struct SceneRecords {
       ck(rtb_scene_set_perlin(s, (uint32_t)i, perlins[i]->ranvec.data(), perlins[i]->perm_x.data(), perlins[i]->perm_y.data(), perlins[i]->perm_z.data()));
     for (size_t i = 0; i < meshes.size(); ++i)
       ck(rtb_scene_set_mesh(s, (uint32_t)i, meshes[i]->vertices.data(), (uint32_t)(meshes[i]->vertices.size() / 3), meshes[i]->indices.data(), (uint32_t)(meshes[i]->indices.size() / 3)));
+    for (size_t i = 0; i < meshes.size(); ++i) {
+      const TriangleMesh& m = *meshes[i];
+      if (m.normals.empty() && m.uvs.empty()) continue;
+      auto ptr = [](const auto& v) { return v.empty() ? nullptr : v.data(); };
+      ck(rtb_scene_set_mesh_attributes(s, (uint32_t)i, ptr(m.normals), (uint32_t)(m.normals.size() / 3), ptr(m.normal_indices),
+                                       ptr(m.uvs), (uint32_t)(m.uvs.size() / 2), ptr(m.uv_indices)));
+    }
     ck(rtb_scene_set_lights(s, lights.empty() ? nullptr : lights.data(), (uint32_t)lights.size()));
     ck(rtb_scene_set_graph(s, nodes.data(), (uint32_t)nodes.size(), child_index.data(), (uint32_t)child_index.size(), root));
   }

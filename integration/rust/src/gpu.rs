@@ -142,6 +142,10 @@ extern "C" {
     pub fn rtb_scene_set_image(s: *mut RtbScene, id: u32, rgb: *const u8, w: u32, h: u32) -> c_int;
     pub fn rtb_scene_set_perlin(s: *mut RtbScene, id: u32, ranvec: *const f64, px: *const u32, py: *const u32, pz: *const u32) -> c_int;
     pub fn rtb_scene_set_mesh(s: *mut RtbScene, id: u32, verts: *const f32, nv: u32, idx: *const u32, nt: u32) -> c_int;
+    // vertex normals / texture coordinates of mesh `id` (NULL data: no such stream; NULL indices: the position indices)
+    pub fn rtb_scene_set_mesh_attributes(s: *mut RtbScene, id: u32, normals: *const f32, n_normals: u32,
+                                         normal_idx: *const u32, uvs: *const f32, n_uvs: u32, uv_idx: *const u32) -> c_int;
+    pub fn rtb_scene_export_triangle_attributes(s: *mut RtbScene, records: *mut f32, cap_bytes: usize) -> c_int;
     pub fn rtb_scene_set_lights(s: *mut RtbScene, l: *const RtbLight, n: u32) -> c_int;
     pub fn rtb_scene_set_graph(s: *mut RtbScene, nodes: *const RtbNode, n: u32, child: *const u32, nc: u32, root: u32) -> c_int;
     pub fn rtb_scene_build_bvh(s: *mut RtbScene) -> c_int;

@@ -106,6 +106,7 @@ SIGNATURES = {
     "rtb_scene_set_image": (_I, [_VP, _U32, _VP, _U32, _U32]),
     "rtb_scene_set_perlin": (_I, [_VP, _U32, _VP, _VP, _VP, _VP]),
     "rtb_scene_set_mesh": (_I, [_VP, _U32, _VP, _U32, _VP, _U32]),
+    "rtb_scene_set_mesh_attributes": (_I, [_VP, _U32, _VP, _U32, _VP, _VP, _U32, _VP]),
     "rtb_scene_set_lights": (_I, [_VP, _VP, _U32]),
     "rtb_scene_set_graph": (_I, [_VP, _VP, _U32, _VP, _U32, _U32]),
     "rtb_scene_set_spheres": (_I, [_VP, _VP, _VP, _VP, _VP, _U32]),
@@ -121,6 +122,7 @@ SIGNATURES = {
     "rtb_scene_export_globals": (_I, [_VP, _VP, _U32, C.POINTER(C.c_uint32)]),
     "rtb_scene_export_prims": (_I, [_VP, _U32, _VP, _SZ, _VP, _SZ]),
     "rtb_scene_export_exact": (_I, [_VP, _U32, _VP, _SZ, C.POINTER(C.c_float), C.POINTER(C.c_float)]),
+    "rtb_scene_export_triangle_attributes": (_I, [_VP, _VP, _SZ]),
     "rtb_render": (_I, [_VP, _VP, C.POINTER(Camera), C.POINTER(Params), _VP, C.POINTER(Stats)]),
     "rtb_render_device": (_I, [_VP, _VP, C.POINTER(Camera), C.POINTER(Params), _VP, _VP, C.POINTER(Stats)]),
     "rtb_render_aov": (_I, [_VP, _VP, C.POINTER(Camera), C.POINTER(Params), _VP, C.POINTER(Stats)]),

@@ -483,6 +483,7 @@ struct Assembler {
 int build_bvh8(const HostScene& hs, HostBvh& out, std::string& err) {
   out.nodes.clear();
   for (int t = 0; t < (int)PT_COUNT; ++t) { out.geom[t].clear(); out.info[t].clear(); }
+  out.attr.clear();
   out.max_depth = 0;
   out.global_refs.clear();
   const size_t np = hs.prims.size();
@@ -497,6 +498,29 @@ int build_bvh8(const HostScene& hs, HostBvh& out, std::string& err) {
       return RTB_ERR_INVALID;
     }
   }
+
+  // Leaf entries: geometry words, (prim id, material word) and — when some triangle has vertex normals or texture
+  // coordinates — a shading record per triangle (all zero for the flat ones).  Info bit 31 marks a quad with an exact
+  // plane or a triangle with a shading record.
+  bool with_attr = false;
+  for (size_t i = 0; i < np && !with_attr; ++i) with_attr = hs.prims[i].type == PT_TRI && hs.prims[i].attr != RTB_NONE;
+  for (size_t i = 0; i < np; ++i)
+    if (hs.prims[i].type == PT_TRI && hs.prims[i].attr != RTB_NONE && hs.prims[i].attr >= hs.attrs.size()) {
+      err = "internal: triangle shading record out of range";
+      return RTB_ERR_INVALID;
+    }
+  auto emit_leaf = [&](const HostPrim& p, std::vector<float>* geom, std::vector<uint32_t>* info, std::vector<float>& attr) {
+    for (uint32_t w = 0; w < geom_words(p.type); ++w) geom[p.type].push_back(p.g[w]);
+    const bool has_attr = p.type == PT_TRI && p.attr != RTB_NONE;
+    info[p.type].push_back(p.prim_id);
+    info[p.type].push_back((p.material & 0xFFFFFFu) | (p.face_mode << 24) |
+                           ((p.type == PT_QUAD && p.plane_exact) || has_attr ? 0x80000000u : 0u));
+    if (with_attr && p.type == PT_TRI) {
+      static const AttrRec flat{};
+      const AttrRec& r = has_attr ? hs.attrs[p.attr] : flat;
+      attr.insert(attr.end(), r.f, r.f + RTB_ATTR_FLOATS);
+    }
+  };
 
   // --- "global" primitives: a primitive whose box is (nearly) the whole scene box (the r=1000 ground sphere of
   // book 1) cannot be culled by any node and only coarsens the quantisation grid of the node that holds
@@ -591,9 +615,7 @@ int build_bvh8(const HostScene& hs, HostBvh& out, std::string& err) {
       if (!is_global[i]) continue;
       const HostPrim& p = hs.prims[i];
       const uint32_t idx = (uint32_t)(out.info[p.type].size() / 2);
-      for (uint32_t w = 0; w < geom_words(p.type); ++w) out.geom[p.type].push_back(p.g[w]);
-      out.info[p.type].push_back(p.prim_id);
-      out.info[p.type].push_back((p.material & 0xFFFFFFu) | (p.face_mode << 24) | (p.type == PT_QUAD && p.plane_exact ? 0x80000000u : 0u));
+      emit_leaf(p, out.geom, out.info, out.attr);
       out.global_refs.push_back((p.type << REF_TYPE_SHIFT) | idx);
     }
   };
@@ -679,6 +701,7 @@ int build_bvh8(const HostScene& hs, HostBvh& out, std::string& err) {
     std::vector<Node8>* nodes;
     std::vector<float>* geom;      // [PT_COUNT]
     std::vector<uint32_t>* info;   // [PT_COUNT]
+    std::vector<float>* attr;      // triangle shading records
     std::vector<Pending>* queue;
     uint32_t max_depth = 0;
   };
@@ -732,7 +755,6 @@ int build_bvh8(const HostScene& hs, HostBvh& out, std::string& err) {
     Node8 n;
     std::memset(&n, 0, sizeof(n));
     as.quantise(n, ch, slot_of, nc);
-    const uint32_t gw = geom_words(type);
     const uint32_t prim_base = (uint32_t)(sk.info[type].size() / 2);
     if (prim_base > REF_INDEX_MASK) { perr = "too many primitives of one type"; return false; }
     n.prim_base = (type << REF_TYPE_SHIFT) | prim_base;
@@ -746,10 +768,7 @@ int build_bvh8(const HostScene& hs, HostBvh& out, std::string& err) {
         if (lf.count > 3 || off + lf.count > 24) { perr = "internal: leaf too large"; return false; }
         n.meta[s] = (uint8_t)((lf.count << 5) | off);
         for (uint32_t q = 0; q < lf.count; ++q) {
-          const HostPrim& p = hs.prims[b.recs[lf.first + q].prim()];
-          for (uint32_t w = 0; w < gw; ++w) sk.geom[type].push_back(p.g[w]);
-          sk.info[type].push_back(p.prim_id);
-          sk.info[type].push_back((p.material & 0xFFFFFFu) | (p.face_mode << 24) | (p.type == PT_QUAD && p.plane_exact ? 0x80000000u : 0u));
+          emit_leaf(hs.prims[b.recs[lf.first + q].prim()], sk.geom, sk.info, *sk.attr);
         }
         off += lf.count;
       } else {
@@ -765,7 +784,7 @@ int build_bvh8(const HostScene& hs, HostBvh& out, std::string& err) {
 
   // Serial breadth-first phase: the top of the tree (at least the prefix the extend kernel stages in shared memory)
   // stays in pure breadth-first order.  Large trees then hand the pending subtrees to worker threads.
-  Sink top{&out.nodes, out.geom, out.info, &queue, 0};
+  Sink top{&out.nodes, out.geom, out.info, &out.attr, &queue, 0};
   const bool parallel = np >= 50000 && !(getenv("RTB_BVH_PAR") && atoi(getenv("RTB_BVH_PAR")) == 0);
   while (qhead < queue.size()) {
     if (parallel && out.nodes.size() >= 1024 && queue.size() - qhead >= 64) break;
@@ -781,6 +800,7 @@ int build_bvh8(const HostScene& hs, HostBvh& out, std::string& err) {
       std::vector<Node8> nodes;
       std::vector<float> geom[PT_COUNT];
       std::vector<uint32_t> info[PT_COUNT];
+      std::vector<float> attr;
       uint32_t max_depth = 0;
       std::string err;
       bool ok = true;
@@ -798,7 +818,7 @@ int build_bvh8(const HostScene& hs, HostBvh& out, std::string& err) {
         sb.nodes.emplace_back();  // local node 0 = the subtree root (its global index was allocated by its parent)
         lq.clear();
         lq.push_back(Pending{0u, root.tree, root.bin_node, root.depth});
-        Sink sk{&sb.nodes, sb.geom, sb.info, &lq, 0};
+        Sink sk{&sb.nodes, sb.geom, sb.info, &sb.attr, &lq, 0};
         for (size_t h = 0; h < lq.size() && sb.ok; ++h) {
           const Pending pd = lq[h];  // copy: process() appends to lq
           sb.ok = process(pd, sk, sb.err);
@@ -829,6 +849,7 @@ int build_bvh8(const HostScene& hs, HostBvh& out, std::string& err) {
       }
       out.geom[type].insert(out.geom[type].end(), sb.geom[type].begin(), sb.geom[type].end());
       out.info[type].insert(out.info[type].end(), sb.info[type].begin(), sb.info[type].end());
+      out.attr.insert(out.attr.end(), sb.attr.begin(), sb.attr.end());  // (triangle subtrees only)
       if (sb.max_depth > out.max_depth) out.max_depth = sb.max_depth;
     }
   }

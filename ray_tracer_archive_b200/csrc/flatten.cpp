@@ -108,6 +108,7 @@ struct Walker {
     p.material = material;
     p.face_mode = face_mode;
     p.exact = RTB_NONE;
+    p.attr = RTB_NONE;
     return p;
   }
 
@@ -237,6 +238,10 @@ struct Walker {
         hs.prims.resize(first + ntri);
         hs.n_prim_ids += (uint32_t)ntri;
         const uint32_t material = n.material;
+        // shading records: one per triangle when the mesh has vertex normals or texture coordinates
+        const bool has_n = !m.normals.empty(), has_uv = !m.uvs.empty();
+        const size_t attr0 = hs.attrs.size();
+        if (has_n || has_uv) hs.attrs.resize(attr0 + ntri);
         auto pack_range = [&](size_t t0, size_t t1) {
           for (size_t t = t0; t < t1; ++t) {
             double v[3][3];
@@ -252,8 +257,34 @@ struct Walker {
             pr.material = material;
             pr.face_mode = fm;
             pr.exact = RTB_NONE;
+            pr.attr = RTB_NONE;
             pack_tri(pr, v[0], v[1], v[2]);
             pr.g[3] = (float)x.s; pr.g[7] = (float)x.c;
+            if (has_n || has_uv) {
+              AttrRec& a = hs.attrs[attr0 + t];
+              std::memset(&a, 0, sizeof(a));
+              uint32_t flags = 0;
+              if (has_n) {  // the vertices' RotateY turns the normals; a Translate leaves them alone
+                for (int q = 0; q < 3; ++q) {
+                  const float* f = &m.normals[3 * (size_t)m.normal_idx[3 * t + q]];
+                  const double d[3] = {f[0], f[1], f[2]};
+                  double w[3];
+                  x.vec(d, w);
+                  for (int c = 0; c < 3; ++c) a.f[4 * q + c] = (float)w[c];
+                }
+                flags |= ATTR_NORMALS;
+              }
+              if (has_uv) {
+                for (int q = 0; q < 3; ++q) {
+                  const float* f = &m.uvs[2 * (size_t)m.uv_idx[3 * t + q]];
+                  a.f[4 * q + 3] = f[0];
+                  a.f[12 + q] = f[1];
+                }
+                flags |= ATTR_UVS;
+              }
+              std::memcpy(&a.f[15], &flags, 4);
+              pr.attr = (uint32_t)(attr0 + t);
+            }
           }
         };
         unsigned n_thr = ntri >= 100000 ? std::max(1u, std::min(std::thread::hardware_concurrency(), 16u)) : 1u;
@@ -478,6 +509,7 @@ int flatten_graph(HostScene& hs, const rtb_node* nodes, uint32_t n_nodes, const 
   hs.prims.clear();
   hs.media.clear();
   hs.exact.clear();
+  hs.attrs.clear();
   hs.n_prim_ids = 0;
   Walker w{hs, nodes, n_nodes, child_index, n_child_index, err};
   Xform id;

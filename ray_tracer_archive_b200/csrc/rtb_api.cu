@@ -109,6 +109,7 @@ struct rtb_scene {
   DevBuf<float4> d_geom[PT_COUNT];
   DevBuf<uint2> d_info[PT_COUNT];
   DevBuf<double> d_exact[PT_COUNT];
+  DevBuf<float4> d_attr;  // leaf-ordered triangle shading records (4 words each), empty without attributes
   DevBuf<ExactTab> d_xtab;
   DevBuf<DevScene> d_self;
   DevBuf<float4> d_materials;
@@ -386,8 +387,55 @@ int rtb_scene_set_mesh(rtb_scene* s, uint32_t id, const float* verts, uint32_t n
   for (size_t i = 0; i < (size_t)nt * 3; ++i)
     if (idx[i] >= nv) return set_err(RTB_ERR_INVALID, "mesh index out of range");
   if (s->hs.meshes.size() <= id) s->hs.meshes.resize(id + 1);
-  s->hs.meshes[id].verts.assign(verts, verts + (size_t)nv * 3);
-  s->hs.meshes[id].idx.assign(idx, idx + (size_t)nt * 3);
+  HostScene::Mesh& m = s->hs.meshes[id];
+  m = HostScene::Mesh();  // (clears the shading attributes of an earlier mesh with this id)
+  m.verts.assign(verts, verts + (size_t)nv * 3);
+  m.idx.assign(idx, idx + (size_t)nt * 3);
+  s->built = s->committed = false;
+  return RTB_OK;
+}
+// one attribute stream of a mesh: `dim` floats per element, per-corner indices (NULL: the position indices)
+static int mesh_stream(const HostScene::Mesh& m, const float* data, uint32_t n, const uint32_t* idx, int dim,
+                       const char* what, std::vector<float>& out_data, std::vector<uint32_t>& out_idx) {
+  out_data.clear();
+  out_idx.clear();
+  if (!data) return RTB_OK;
+  const size_t n_corners = m.idx.size();
+  if (!idx && (size_t)n * 3 != m.verts.size())
+    return set_err(RTB_ERR_INVALID, std::string(what) + " without indices must have one entry per mesh vertex");
+  for (size_t i = 0; i < (size_t)n * dim; ++i)
+    if (!std::isfinite(data[i])) return set_err(RTB_ERR_INVALID, std::string(what) + " must be finite");
+  if (idx)
+    for (size_t i = 0; i < n_corners; ++i)
+      if (idx[i] >= n) return set_err(RTB_ERR_INVALID, std::string(what) + " index out of range");
+  out_data.resize((size_t)n * dim);
+  if (dim == 3) {  // unit normals: normalised in f64, rounded once (a zero normal stays zero: the shading falls back)
+    for (size_t i = 0; i < n; ++i) {
+      const double x = data[3 * i], y = data[3 * i + 1], z = data[3 * i + 2];
+      const double len = std::sqrt(x * x + y * y + z * z);
+      const double k = len > 0.0 ? 1.0 / len : 0.0;
+      out_data[3 * i] = (float)(x * k); out_data[3 * i + 1] = (float)(y * k); out_data[3 * i + 2] = (float)(z * k);
+    }
+  } else {
+    out_data.assign(data, data + (size_t)n * dim);
+  }
+  if (idx) out_idx.assign(idx, idx + n_corners);
+  else out_idx = m.idx;
+  return RTB_OK;
+}
+int rtb_scene_set_mesh_attributes(rtb_scene* s, uint32_t id, const float* normals, uint32_t n_normals,
+                                  const uint32_t* normal_idx, const float* uvs, uint32_t n_uvs, const uint32_t* uv_idx) {
+  if (!s) return set_err(RTB_ERR_INVALID, "scene is NULL");
+  if (id >= s->hs.meshes.size() || s->hs.meshes[id].idx.empty())
+    return set_err(RTB_ERR_INVALID, "mesh id was not set (call rtb_scene_set_mesh first)");
+  HostScene::Mesh& m = s->hs.meshes[id];
+  std::vector<float> nd, ud;
+  std::vector<uint32_t> ni, ui;
+  int rc = mesh_stream(m, normals, n_normals, normal_idx, 3, "normals", nd, ni);
+  if (rc == RTB_OK) rc = mesh_stream(m, uvs, n_uvs, uv_idx, 2, "uvs", ud, ui);
+  if (rc != RTB_OK) return rc;
+  m.normals.swap(nd); m.normal_idx.swap(ni);
+  m.uvs.swap(ud); m.uv_idx.swap(ui);
   s->built = s->committed = false;
   return RTB_OK;
 }
@@ -435,6 +483,7 @@ static HostPrim& add_flat(rtb_scene* s, uint32_t type, const uint32_t* mat, cons
   p.material = mat[i];
   p.face_mode = flags ? face_mode_of(flags[i]) : FACE_NATURAL;
   p.exact = RTB_NONE;
+  p.attr = RTB_NONE;
   p.prim_id = id ? id[i] : s->hs.n_prim_ids;
   s->hs.n_prim_ids = std::max(s->hs.n_prim_ids, p.prim_id + 1);
   return p;
@@ -745,6 +794,10 @@ static int upload_scene(rtb_scene* s, const rtb_scene* host) {
     for (int t = 0; t < 3; ++t) xt.exact[t] = s->d_exact[t].p;
     for (uint32_t t = 0; t < PT_COUNT; ++t) xt.info[t] = s->d_info[t].p;
     for (size_t i = 0; i < hs.media.size() && i < RTB_MAX_MEDIA; ++i) xt.media_prim_id[i] = hs.media[i].prim_id;
+    if (bvh.attr.empty()) s->d_attr.release();  // (allocated only for a scene with shading records)
+    else CU(s->d_attr.upload(reinterpret_cast<const float4*>(bvh.attr.data()), bvh.attr.size() / 4));
+    xt.attr = s->d_attr.p;
+    xt.n_attr = (uint32_t)(bvh.attr.size() / RTB_ATTR_FLOATS);
     CU(s->d_xtab.upload(&xt, 1));
     CU(cudaStreamSynchronize(0));  // `xt` is a temporary
     d.xtab = s->d_xtab.p;
@@ -754,6 +807,7 @@ static int upload_scene(rtb_scene* s, const rtb_scene* host) {
   CU(cudaMemcpy(s->d_self.p, &d, sizeof(DevScene), cudaMemcpyHostToDevice));  // (after every other field is final)
   int e = configure_launch(s->lc, d.n_nodes, s->bvh.max_depth, d.n_prims[PT_SPHERE], s->ctx->prop.multiProcessorCount);
   if (e != 0) return set_err(RTB_ERR_CUDA, std::string("configure_launch: ") + cudaGetErrorString((cudaError_t)e));
+  s->lc.attr = !bvh.attr.empty();
   CU(cudaStreamSynchronize(0));
   s->committed = true;
   return RTB_OK;
@@ -821,6 +875,15 @@ int rtb_scene_export_exact(rtb_scene* s, uint32_t type, double* out, size_t cap_
   if (out && bytes) std::memcpy(out, s->bvh.exact[type].data(), bytes);
   if (coord_max) *coord_max = s->bvh.coord_max;
   if (eps_ab) *eps_ab = s->bvh.eps_ab;
+  return RTB_OK;
+}
+int rtb_scene_export_triangle_attributes(rtb_scene* s, float* records, size_t cap_bytes) {
+  if (!s || !records) return set_err(RTB_ERR_INVALID, "NULL argument");
+  if (!s->built) return set_err(RTB_ERR_STATE, "BVH not built (call rtb_scene_build_bvh or rtb_scene_commit)");
+  const size_t n = s->bvh.info[PT_TRI].size() / 2, bytes = n * RTB_ATTR_FLOATS * sizeof(float);
+  if (cap_bytes < bytes) return set_err(RTB_ERR_INVALID, "buffer too small");
+  if (s->bvh.attr.empty()) std::memset(records, 0, bytes);
+  else std::memcpy(records, s->bvh.attr.data(), bytes);
   return RTB_OK;
 }
 int rtb_scene_export_prims(rtb_scene* s, uint32_t type, float* geom, size_t gcap, uint32_t* info, size_t icap) {
@@ -1300,7 +1363,7 @@ int rtb_render_aov_device(rtb_context* c, rtb_scene* s, const rtb_camera* cam, c
     launch_aov_fill(pool[k], prm, dcam, first, n, ls);
     launch_extend(s->lc, s->dev, pool[k], prm, false, ls);
     launch_fixup(s->lc, s->dev, pool[k], prm, ls);
-    launch_aov_collect(s->dev, pool[k], prm, aov, n, ls);
+    launch_aov_collect(s->lc, s->dev, pool[k], prm, aov, n, ls);
     launches += 4;
     extend_launches += 1;
     first += n;

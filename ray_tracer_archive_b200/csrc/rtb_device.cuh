@@ -17,7 +17,7 @@ namespace rtb {
 // (rtb_debug_check_failures) instead of trapping, so one run reports everything.
 #ifdef RTB_CHECKED
 __device__ unsigned int g_rtb_check_fail[8];
-enum CheckKind : int { CHK_STACK = 0, CHK_NODE = 1, CHK_PRIM = 2, CHK_SLOT = 3, CHK_QUEUE = 4, CHK_LIST = 5 };
+enum CheckKind : int { CHK_STACK = 0, CHK_NODE = 1, CHK_PRIM = 2, CHK_SLOT = 3, CHK_QUEUE = 4, CHK_LIST = 5, CHK_ATTR = 6 };
 #define RTB_CHECK(kind, cond)                          \
   do {                                                 \
     if (!(cond)) atomicAdd(&g_rtb_check_fail[kind], 1u); \
@@ -35,7 +35,8 @@ enum CheckKind : int { CHK_STACK = 0, CHK_NODE = 1, CHK_PRIM = 2, CHK_SLOT = 3, 
 #define RTB_PI 3.14159265358979323846f
 
 enum Queue : uint32_t { Q_TERMINAL = 0, Q_LAMBERT = 1, Q_METAL = 2, Q_DIELECTRIC = 3, Q_ISOTROPIC = 4, Q_COUNT = 5 };
-// per-primitive info word y (device copy): material (24 bits) | face mode << 24 (4 bits, FaceMode) | shade queue << 28 (3 bits) | bit 31: quad with an exact plane.
+// per-primitive info word y (device copy): material (24 bits) | face mode << 24 (4 bits, FaceMode) | shade queue << 28 (3 bits) | bit 31: quad with an exact plane,
+// triangle with a shading record (ExactTab::attr).
 // The queue is resolved from the material type on the host at commit, so `extend` classifies a hit without touching
 // the material table (one dependent load less on its tail).
 #define RTB_MINFO_MAT(m) ((m) & 0xFFFFFFu)
@@ -64,6 +65,8 @@ struct ExactTab {
   const double* exact[3];         // sphere / moving sphere / quad records, RTB_EXACT_STRIDE doubles each
   const uint2* info[PT_COUNT];    // (primitive id, material word) per leaf entry
   uint32_t media_prim_id[RTB_MAX_MEDIA];
+  const float4* attr;             // leaf-ordered triangle shading records, 4 words each (rtb_internal.hpp AttrRec); or NULL
+  uint32_t n_attr;                // records (RTB_CHECKED bounds)
 };
 
 struct DevScene {  // passed by value as a kernel parameter (constant bank)

@@ -34,7 +34,15 @@ struct HostPrim {      // one flattened primitive, any type
   float lo[3], hi[3];  // bounds (padded)
   uint32_t exact;      // index into HostScene::exact (RTB_NONE for triangles: their f32 vertices ARE the exact record)
   uint32_t plane_exact;  // quad: axis-aligned and its plane constant is exactly a float (info word bit 31)
+  uint32_t attr;         // triangle: index into HostScene::attrs (RTB_NONE: flat shading)
 };
+
+// Shading record of a mesh triangle with vertex normals and / or texture coordinates (rtb_scene_set_mesh_attributes),
+// 16 floats: [0..2] n0 [3] u0 [4..6] n1 [7] u1 [8..10] n2 [11] u2 [12] v0 [13] v1 [14] v2 [15] flags (bits).  Normals are
+// world-space unit vectors.  The device reads it as four float4 words (surface_at<ATTR>, rtb_kernels.cu).
+#define RTB_ATTR_FLOATS 16
+enum AttrFlags : uint32_t { ATTR_NORMALS = 1u, ATTR_UVS = 2u };
+struct AttrRec { float f[RTB_ATTR_FLOATS]; };
 
 // Reference-exact record of one sphere / moving sphere / quad: the constructor's own f64 arguments in OBJECT space plus
 // the wrapper chain the reference evaluates per ray (Translate outside RotateY, hittable.rs:76-85,147-176).  The device
@@ -82,6 +90,8 @@ struct HostBvh {
   std::vector<double> exact[PT_COUNT];
   float coord_max = 0.f, eps_ab = 0.f;
   uint32_t global_f64 = 0;  // bit k: global k is a sphere tested in f64 directly (DevScene::global_f64)
+  // leaf-ordered shading records of the triangles (RTB_ATTR_FLOATS per triangle); empty when no triangle has attributes
+  std::vector<float> attr;
 };
 
 static inline uint32_t geom_words(uint32_t type) { return type == PT_SPHERE ? 4u : (type == PT_MOVING ? 8u : 12u); }
@@ -96,9 +106,15 @@ struct HostScene {
   std::vector<Image> images;
   struct Perlin { std::vector<float> ranvec; std::vector<uint8_t> perm; bool set = false; };  // 256x4 floats, 3x256 bytes
   std::vector<Perlin> perlins;
-  struct Mesh { std::vector<float> verts; std::vector<uint32_t> idx; };
+  // normals: unit f32 vectors (normalised in f64) and their per-corner indices; uvs likewise (empty: no such stream)
+  struct Mesh {
+    std::vector<float> verts; std::vector<uint32_t> idx;
+    std::vector<float> normals; std::vector<uint32_t> normal_idx;
+    std::vector<float> uvs; std::vector<uint32_t> uv_idx;
+  };
   std::vector<Mesh> meshes;
   std::vector<ExactRec> exact;
+  std::vector<AttrRec> attrs;  // shading records of mesh triangles (HostPrim::attr)
   uint32_t n_prim_ids = 0;
   // BVH builder quality knobs (rtb_scene_set_build_options)
   uint32_t opt_max_leaf_tris = 2;   // triangles per leaf slot, 1..3

@@ -709,8 +709,50 @@ struct Surf {
   float3 p, n, outward;  // n = normal against the ray (set_face_normal, hittable.rs:41-48)
   bool front;
   uint32_t mat, ref;
+  bool uv;               // ATTR kernels: (tu, tv) are the texture coordinates of a triangle's shading record
+  float tu, tv;
 };
 
+// barycentrics (u, v) of the point p in the triangle (v0, v0 + e1, v0 + e2): the (u, v) a triangle reports
+__device__ __forceinline__ void tri_bary(float3 v0, float3 e1, float3 e2, float3 p, float& u, float& v) {
+  const float3 nn = cross(e1, e2), pl = p - v0;
+  const float inv = 1.0f / dot(nn, nn);
+  u = dot(nn, cross(pl, e2)) * inv;
+  v = dot(nn, cross(e1, pl)) * inv;
+}
+
+// Shading record of a mesh triangle (info bit 31 in an ATTR kernel; include/rtb200.h rtb_scene_set_mesh_attributes):
+// ns = normalize(b0 n0 + b1 n1 + b2 n2) turned to the side of the ray-facing geometric normal s.n, which it then replaces
+// (front_face stays the geometric one: surface_at has decided it); (u, v) interpolated the same way.  A non-finite or
+// near-zero interpolated normal keeps the geometric one.  No bending towards the geometric surface (DESIGN.md §9).
+__device__ __forceinline__ void surface_attr(const DevScene& sc, uint32_t idx, Surf& s) {
+  RTB_CHECK(CHK_ATTR, idx < sc.xtab->n_attr);
+  const float4* rec = sc.xtab->attr + 4 * (size_t)idx;
+  const float3 v0 = xyz(__ldg(sc.geom[PT_TRI] + 3 * idx)), e1 = xyz(__ldg(sc.geom[PT_TRI] + 3 * idx + 1)) - v0,
+               e2 = xyz(__ldg(sc.geom[PT_TRI] + 3 * idx + 2)) - v0;
+  float b1, b2;
+  tri_bary(v0, e1, e2, s.p, b1, b2);
+  const float b0 = 1.0f - b1 - b2;
+  const float4 w0 = __ldg(rec), w1 = __ldg(rec + 1), w2 = __ldg(rec + 2), w3 = __ldg(rec + 3);
+  const uint32_t flags = __float_as_uint(w3.w);
+  if (flags & ATTR_NORMALS) {
+    const float3 sum = fma3(b0, xyz(w0), fma3(b1, xyz(w1), b2 * xyz(w2)));
+    const float len2 = dot(sum, sum);
+    if (isfinite(len2) && len2 >= 1e-20f) {
+      const float3 ns = rsqrtf(len2) * sum;
+      s.n = dot(ns, s.n) < 0.0f ? -ns : ns;
+    }
+  }
+  if (flags & ATTR_UVS) {
+    s.uv = true;
+    s.tu = fmaf(b0, w0.w, fmaf(b1, w1.w, b2 * w2.w));
+    s.tv = fmaf(b0, w3.x, fmaf(b1, w3.y, b2 * w3.z));
+  }
+}
+
+// ATTR: the scene has triangles with shading records (rtb_scene_set_mesh_attributes); the kernels of other scenes are
+// compiled without that path
+template <bool ATTR = false>
 __device__ __forceinline__ Surf surface_at(const DevScene& sc, uint32_t ref, uint32_t minfo, float3 o, float3 d, float time, float t) {
   Surf s;
   s.ref = ref;
@@ -755,10 +797,18 @@ __device__ __forceinline__ Surf surface_at(const DevScene& sc, uint32_t ref, uin
   } else {
     s.front = base == FACE_NATURAL ? ff : base == FACE_FLIPPED ? !ff : base == FACE_TRUE;
   }
+  if constexpr (ATTR) {
+    s.uv = false;
+    if (type == PT_TRI && (minfo >> 31)) surface_attr(sc, idx, s);
+  }
   return s;
 }
 
+template <bool ATTR = false>
 __device__ __forceinline__ void surface_uv(const DevScene& sc, const Surf& s, float& u, float& v) {
+  if constexpr (ATTR) {
+    if (s.uv) { u = s.tu; v = s.tv; return; }
+  }
   const uint32_t type = s.ref >> REF_TYPE_SHIFT, idx = s.ref & REF_INDEX_MASK;
   u = v = 0.f;  // MovingSphere / ConstantMedium leave u,v stale in the reference; defined 0 (SURVEY App. A #17)
   if (type == PT_SPHERE) {  // sphere.rs:32-37, on the OBJECT-space outward normal: a sphere under RotateY gets its
@@ -777,10 +827,7 @@ __device__ __forceinline__ void surface_uv(const DevScene& sc, const Surf& s, fl
   } else if (type == PT_TRI) {
     const float3 v0 = xyz(__ldg(sc.geom[PT_TRI] + 3 * idx)), e1 = xyz(__ldg(sc.geom[PT_TRI] + 3 * idx + 1)) - v0,
                  e2 = xyz(__ldg(sc.geom[PT_TRI] + 3 * idx + 2)) - v0;
-    const float3 nn = cross(e1, e2), pl = s.p - v0;
-    const float inv = 1.0f / dot(nn, nn);
-    u = dot(nn, cross(pl, e2)) * inv;
-    v = dot(nn, cross(e1, pl)) * inv;
+    tri_bary(v0, e1, e2, s.p, u, v);
   }
 }
 
@@ -819,6 +866,7 @@ __device__ float perlin_turb(const float4* __restrict__ vec, const uint8_t* __re
   return fabsf(accum);
 }
 
+template <bool ATTR = false>
 __device__ float3 tex_value_slow(const DevScene& sc, uint32_t tex, const Surf& s) {
   DevTexture t = sc.textures[tex];
   if (t.type == RTB_TEX_CHECKER) {  // texture.rs:60-69, on the world-space point
@@ -835,7 +883,7 @@ __device__ float3 tex_value_slow(const DevScene& sc, uint32_t tex, const Surf& s
     const DevImage im = sc.images[t.table];
     if (im.data == nullptr) return f3(0.f, 1.f, 1.f);
     float u, v;
-    surface_uv(sc, s, u, v);
+    surface_uv<ATTR>(sc, s, u, v);
     u = fminf(fmaxf(u, 0.f), 1.f);
     v = 1.0f - fminf(fmaxf(v, 0.f), 1.f);
     uint32_t i = (uint32_t)(u * (float)im.w), j = (uint32_t)(v * (float)im.h);
@@ -849,9 +897,10 @@ __device__ float3 tex_value_slow(const DevScene& sc, uint32_t tex, const Surf& s
 }
 
 // material word 0 = (type, texture, param, texture type); word 1 = solid albedo (saves the texture fetch)
+template <bool ATTR = false>
 __device__ __forceinline__ float3 tex_value(const DevScene& sc, const float4 m0, uint32_t mat, const Surf& s) {
   if (__float_as_uint(m0.w) == RTB_TEX_SOLID) return xyz(__ldg(&sc.materials[2 * mat + 1]));
-  return tex_value_slow(sc, __float_as_uint(m0.y), s);
+  return tex_value_slow<ATTR>(sc, __float_as_uint(m0.y), s);
 }
 
 struct Onb {  // onb.rs:19-42
@@ -1063,6 +1112,7 @@ __device__ __forceinline__ void shade_loop(const DevPool& pool, const DevParams&
 }
 
 // miss -> background (main.rs:74-76); DiffuseLight -> emitted iff front_face, no scatter (material.rs:184-190, main.rs:85-87)
+template <bool ATTR>
 __global__ void __launch_bounds__(RTB_SHADE_THREADS, RTB_SHADE_MIN_BLOCKS) k_shade_terminal(DevScene sc, DevPool pool, DevParams prm, DevCamera cam) {
   shade_loop<Q_TERMINAL>(pool, prm, cam, [&](uint32_t slot) {
     // a miss needs only the throughput/radiance sector; the ray is fetched for emitters alone
@@ -1074,22 +1124,24 @@ __global__ void __launch_bounds__(RTB_SHADE_THREADS, RTB_SHADE_MIN_BLOCKS) k_sha
       L = L + beta * f3(prm.bg[0], prm.bg[1], prm.bg[2]);
     } else {
       const float4 ro = pool.ray[2 * slot], rd = pool.ray[2 * slot + 1];
-      const Surf s = surface_at(sc, ref, __float_as_uint(h.z), xyz(ro), xyz(rd), ro.w, h.x);
+      const Surf s = surface_at<ATTR>(sc, ref, __float_as_uint(h.z), xyz(ro), xyz(rd), ro.w, h.x);
       const float4 m = __ldg(&sc.materials[2 * s.mat]);
-      if (__float_as_uint(m.x) == RTB_MAT_DIFFUSE_LIGHT && s.front) L = L + beta * tex_value(sc, m, s.mat, s);
+      if (__float_as_uint(m.x) == RTB_MAT_DIFFUSE_LIGHT && s.front) L = L + beta * tex_value<ATTR>(sc, m, s.mat, s);
     }
     deposit(prm, pool.c, __float_as_uint(b.w), L);
     return false;
   });
 }
+// (instantiated here: the ATTR = false kernels keep their place, and so their code, in the module)
+template __global__ void k_shade_terminal<false>(DevScene, DevPool, DevParams, DevCamera);
 
 // Lambertian (material.rs:48-71) / Isotropic (SURVEY §8a M6) through the mixture pdf of main.rs:94-138
-template <bool ISO>
+template <bool ISO, bool ATTR>
 __device__ __forceinline__ bool shade_diffuse(const DevScene& sc, const DevPool& pool, const DevParams& prm, uint32_t slot) {
   PathIO io = load_path(pool, slot);
-  const Surf s = surface_at(sc, io.ref, io.minfo, io.o, io.d, io.time, io.t);
+  const Surf s = surface_at<ATTR>(sc, io.ref, io.minfo, io.o, io.d, io.time, io.t);
   const float4 m = __ldg(&sc.materials[2 * s.mat]);
-  const float3 atten = tex_value(sc, m, s.mat, s);
+  const float3 atten = tex_value<ATTR>(sc, m, s.mat, s);
   const float4 us = philox_u(io.pixel, io.sample, BLK_SCATTER, io.segs, prm.seed);
   const bool have_lights = sc.n_lights > 0;
   float3 dir;
@@ -1124,23 +1176,28 @@ __device__ __forceinline__ bool shade_diffuse(const DevScene& sc, const DevPool&
   return finish_bounce(pool, prm, io, scattered, s.p, dir, io.time, rr);
 }
 
+template <bool ATTR>
 __global__ void __launch_bounds__(RTB_SHADE_THREADS, RTB_SHADE_MIN_BLOCKS) k_shade_lambert(DevScene sc, DevPool pool, DevParams prm, DevCamera cam) {
-  shade_loop<Q_LAMBERT>(pool, prm, cam, [&](uint32_t slot) { return shade_diffuse<false>(sc, pool, prm, slot); });
+  shade_loop<Q_LAMBERT>(pool, prm, cam, [&](uint32_t slot) { return shade_diffuse<false, ATTR>(sc, pool, prm, slot); });
 }
+template __global__ void k_shade_lambert<false>(DevScene, DevPool, DevParams, DevCamera);
 
+template <bool ATTR>
 __global__ void __launch_bounds__(RTB_SHADE_THREADS, RTB_SHADE_MIN_BLOCKS) k_shade_isotropic(DevScene sc, DevPool pool, DevParams prm, DevCamera cam) {
-  shade_loop<Q_ISOTROPIC>(pool, prm, cam, [&](uint32_t slot) { return shade_diffuse<true>(sc, pool, prm, slot); });
+  shade_loop<Q_ISOTROPIC>(pool, prm, cam, [&](uint32_t slot) { return shade_diffuse<true, ATTR>(sc, pool, prm, slot); });
 }
+template __global__ void k_shade_isotropic<false>(DevScene, DevPool, DevParams, DevCamera);
 
 // The two specular materials share one kernel (their classes are small: 10 % and 7 % of C1's hits; as separate kernels
 // each paid a launch, a scan of the class bytes and a tail, profiles/r2e_ncu_summary.md).  A chunk's metal slots come
 // first in the warp's list, then its glass slots, so only one round per chunk mixes the two branches.
 //   Metal::scatter, material.rs:95-107: reflect(unit(d), n) + fuzz * (uniform ball); specular; ray time reset to 0
 //   Dielectric::scatter, material.rs:123-155 (+ reflectance :118-122, refract vec3.rs:246-251)
+template <bool ATTR>
 __global__ void __launch_bounds__(RTB_SHADE_THREADS, RTB_SHADE_MIN_BLOCKS) k_shade_specular(DevScene sc, DevPool pool, DevParams prm, DevCamera cam) {
   shade_loop<Q_METAL, Q_DIELECTRIC>(pool, prm, cam, [&](uint32_t slot) {
       PathIO io = load_path(pool, slot);
-      const Surf s = surface_at(sc, io.ref, io.minfo, io.o, io.d, io.time, io.t);
+      const Surf s = surface_at<ATTR>(sc, io.ref, io.minfo, io.o, io.d, io.time, io.t);
       const float4 m = __ldg(&sc.materials[2 * s.mat]);
       const float3 ud = unit(io.d);
       const float4 ua = philox_u(io.pixel, io.sample, BLK_AUX, io.segs, prm.seed);
@@ -1156,7 +1213,7 @@ __global__ void __launch_bounds__(RTB_SHADE_THREADS, RTB_SHADE_MIN_BLOCKS) k_sha
           __sincosf(phi, &sn, &cs);
           dir = fma3(fuzz * rad, f3(r * cs, r * sn, z), dir);
         }
-        io.beta = io.beta * tex_value(sc, m, s.mat, s);
+        io.beta = io.beta * tex_value<ATTR>(sc, m, s.mat, s);
         ntime = 0.0f;  // material.rs:101
       } else {
         const float ir = m.z;
@@ -1173,6 +1230,7 @@ __global__ void __launch_bounds__(RTB_SHADE_THREADS, RTB_SHADE_MIN_BLOCKS) k_sha
       return finish_bounce(pool, prm, io, true, s.p, dir, ntime, ua.x);
   });
 }
+template __global__ void k_shade_specular<false>(DevScene, DevPool, DevParams, DevCamera);
 
 // ---- generate: initial fill — every chunk starts its first paths (afterwards slots are restarted inside shade_loop) ----
 __global__ void __launch_bounds__(RTB_SHADE_THREADS) k_generate(DevPool pool, DevParams prm, DevCamera cam) {
@@ -1310,6 +1368,7 @@ __global__ void k_aov_fill(DevPool pool, DevParams prm, DevCamera cam, unsigned 
 }
 
 // per-sample (albedo, coverage) and (shading normal, depth) of the hit record, summed into aov[2 pixel], aov[2 pixel + 1]
+template <bool ATTR>
 __global__ void __launch_bounds__(RTB_SHADE_THREADS) k_aov_collect(DevScene sc, DevPool pool, DevParams prm, float4* aov,
                                                                   uint32_t n) {
   const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -1320,12 +1379,12 @@ __global__ void __launch_bounds__(RTB_SHADE_THREADS) k_aov_collect(DevScene sc, 
   float cover = 0.f, depth = 0.f;
   if (ref != REF_MISS) {
     const float4 ro = pool.ray[2 * i], rd = pool.ray[2 * i + 1];
-    const Surf s = surface_at(sc, ref, __float_as_uint(h.z), xyz(ro), xyz(rd), ro.w, h.x);
+    const Surf s = surface_at<ATTR>(sc, ref, __float_as_uint(h.z), xyz(ro), xyz(rd), ro.w, h.x);
     const float4 m = __ldg(&sc.materials[2 * s.mat]);
     const uint32_t type = __float_as_uint(m.x);
     if (type == RTB_MAT_DIELECTRIC) albedo = f3(1.f, 1.f, 1.f);
     else if (type == RTB_MAT_DIFFUSE_LIGHT && !s.front) albedo = f3(0.f, 0.f, 0.f);
-    else albedo = tex_value(sc, m, s.mat, s);
+    else albedo = tex_value<ATTR>(sc, m, s.mat, s);
     if ((ref >> REF_TYPE_SHIFT) != PT_MEDIUM) n3 = s.n;
     cover = 1.f;
     depth = h.x * sqrtf(dot(xyz(rd), xyz(rd)));
@@ -1339,6 +1398,7 @@ __global__ void __launch_bounds__(RTB_SHADE_THREADS) k_aov_collect(DevScene sc, 
   red_add_v4(aov + 2 * (size_t)pixel, albedo.x, albedo.y, albedo.z, cover);
   red_add_v4(aov + 2 * (size_t)pixel + 1, n3.x, n3.y, n3.z, depth);
 }
+template __global__ void k_aov_collect<false>(DevScene, DevPool, DevParams, float4*, uint32_t);
 
 // pixel-centre primary rays, generated in f64 like the reference's camera (camera.rs:60-70) and rounded once
 __global__ void k_primary_rays(DevCameraF64 cam, uint32_t W, uint32_t H, float* __restrict__ org, float* __restrict__ dir,
@@ -1518,13 +1578,19 @@ void launch_extend(const LaunchCfg& lc, const DevScene& sc, const DevPool& pool,
 }
 // The per-material kernels of one iteration run back to back on the lane's stream; they touch disjoint slots (each
 // slot has exactly one class per iteration) and each chunk's path cursor is updated by one warp per kernel.
+template <bool ATTR>
+static void launch_shade_kernels(const LaunchCfg& lc, const DevScene& sc, const DevPool& pool, const DevParams& prm,
+                                 const DevCamera& cam, uint32_t present, cudaStream_t st) {
+  k_shade_terminal<ATTR><<<lc.shade_grid, RTB_SHADE_THREADS, 0, st>>>(sc, pool, prm, cam);
+  if (present & (1u << RTB_MAT_LAMBERTIAN)) k_shade_lambert<ATTR><<<lc.shade_grid, RTB_SHADE_THREADS, 0, st>>>(sc, pool, prm, cam);
+  if (present & ((1u << RTB_MAT_METAL) | (1u << RTB_MAT_DIELECTRIC)))
+    k_shade_specular<ATTR><<<lc.shade_grid, RTB_SHADE_THREADS, 0, st>>>(sc, pool, prm, cam);
+  if (present & (1u << RTB_MAT_ISOTROPIC)) k_shade_isotropic<ATTR><<<lc.shade_grid, RTB_SHADE_THREADS, 0, st>>>(sc, pool, prm, cam);
+}
 void launch_shade(const LaunchCfg& lc, const DevScene& sc, const DevPool& pool, const DevParams& prm,
                   const DevCamera& cam, uint32_t present, cudaStream_t st) {
-  k_shade_terminal<<<lc.shade_grid, RTB_SHADE_THREADS, 0, st>>>(sc, pool, prm, cam);
-  if (present & (1u << RTB_MAT_LAMBERTIAN)) k_shade_lambert<<<lc.shade_grid, RTB_SHADE_THREADS, 0, st>>>(sc, pool, prm, cam);
-  if (present & ((1u << RTB_MAT_METAL) | (1u << RTB_MAT_DIELECTRIC)))
-    k_shade_specular<<<lc.shade_grid, RTB_SHADE_THREADS, 0, st>>>(sc, pool, prm, cam);
-  if (present & (1u << RTB_MAT_ISOTROPIC)) k_shade_isotropic<<<lc.shade_grid, RTB_SHADE_THREADS, 0, st>>>(sc, pool, prm, cam);
+  if (lc.attr) launch_shade_kernels<true>(lc, sc, pool, prm, cam, present, st);
+  else launch_shade_kernels<false>(lc, sc, pool, prm, cam, present, st);
 }
 void launch_finalize(const float4* accum, uint8_t* rgb, uint32_t npix, float inv_spp, cudaStream_t st) {
   k_finalize<<<cdiv(npix, 256), 256, 0, st>>>(accum, rgb, npix, inv_spp);
@@ -1549,9 +1615,10 @@ void launch_aov_fill(const DevPool& pool, const DevParams& prm, const DevCamera&
                      uint32_t n, cudaStream_t st) {
   k_aov_fill<<<cdiv(pool.n_chunks * RTB_CHUNK, 256), 256, 0, st>>>(pool, prm, cam, first_path, n);
 }
-void launch_aov_collect(const DevScene& sc, const DevPool& pool, const DevParams& prm, float4* aov, uint32_t n,
-                        cudaStream_t st) {
-  k_aov_collect<<<cdiv(n, RTB_SHADE_THREADS), RTB_SHADE_THREADS, 0, st>>>(sc, pool, prm, aov, n);
+void launch_aov_collect(const LaunchCfg& lc, const DevScene& sc, const DevPool& pool, const DevParams& prm, float4* aov,
+                        uint32_t n, cudaStream_t st) {
+  if (lc.attr) k_aov_collect<true><<<cdiv(n, RTB_SHADE_THREADS), RTB_SHADE_THREADS, 0, st>>>(sc, pool, prm, aov, n);
+  else k_aov_collect<false><<<cdiv(n, RTB_SHADE_THREADS), RTB_SHADE_THREADS, 0, st>>>(sc, pool, prm, aov, n);
 }
 void launch_primary_rays(const DevCameraF64& cam, uint32_t W, uint32_t H, float* org, float* dir, float* time,
                          cudaStream_t st) {
@@ -1625,7 +1692,7 @@ int configure_launch(LaunchCfg& lc, uint32_t n_nodes, uint32_t max_depth, uint32
   occ = std::min(occ, getenv("RTB_EXTEND_OCC") ? std::max(1, atoi(getenv("RTB_EXTEND_OCC"))) : std::max(1, 512 / RTB_EXTEND_THREADS));
   lc.extend_grid = (uint32_t)(sm_count * occ);
   int occ2 = 0;
-  e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ2, k_shade_lambert, RTB_SHADE_THREADS, 0);
+  e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ2, k_shade_lambert<false>, RTB_SHADE_THREADS, 0);
   if (e != cudaSuccess) return (int)e;
   if (occ2 < 1) occ2 = 1;
   if (getenv("RTB_SHADE_OCC")) occ2 = std::max(1, std::min(occ2, atoi(getenv("RTB_SHADE_OCC"))));

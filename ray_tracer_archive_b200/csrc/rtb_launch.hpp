@@ -42,6 +42,9 @@ struct LaunchCfg {
                              // static kernel; added to extend_smem for that kernel's launch only
   // slots that give every resident shade warp exactly one chunk: pools are sized in multiples of this
   uint32_t pool_unit = 0;
+  // the scene has triangles with shading records: the ATTR instantiations of the shade and AOV kernels read them (set at
+  // commit, after configure_launch)
+  bool attr = false;
 };
 
 // max_depth: levels of the tree (the warp-queue kernel keeps fixed-depth stacks in shared memory)
@@ -63,8 +66,8 @@ void launch_probe_collect(const DevScene& sc, const DevPool& pool, uint32_t n, u
 // then summed as 8 floats per pixel into aov (2 float4 per pixel)
 void launch_aov_fill(const DevPool& pool, const DevParams& prm, const DevCamera& cam, unsigned long long first_path,
                      uint32_t n, cudaStream_t st);
-void launch_aov_collect(const DevScene& sc, const DevPool& pool, const DevParams& prm, float4* aov, uint32_t n,
-                        cudaStream_t st);
+void launch_aov_collect(const LaunchCfg& lc, const DevScene& sc, const DevPool& pool, const DevParams& prm, float4* aov,
+                        uint32_t n, cudaStream_t st);
 void launch_primary_rays(const DevCameraF64& cam, uint32_t W, uint32_t H, float* org, float* dir, float* time,
                          cudaStream_t st);
 void launch_bw_global(const uint4* p, size_t n_vec, uint32_t reps, uint4* sink, uint32_t grid, cudaStream_t st);

@@ -9,29 +9,89 @@ import numpy as np
 from .scene import Material, TriangleMesh
 
 
-def load_obj(path_or_lines, mat: Material, scale: float = 1.0, offset=(0.0, 0.0, 0.0)) -> TriangleMesh:
-    """Wavefront OBJ: `v x y z` and `f a b c ...` (1-based, negative = relative, `a/b/c` forms accepted; polygons are
-    fan-triangulated).  Returns a TriangleMesh for the scene graph (-> rtb_scene_set_mesh)."""
+def load_obj(path_or_lines, mat: Material, scale: float = 1.0, offset=(0.0, 0.0, 0.0), normals=None,
+             uvs: bool = False) -> TriangleMesh:
+    """Wavefront OBJ: `v x y z` and `f a b c ...` (1-based, negative = relative, `a`, `a/t`, `a//n` and `a/t/n` forms
+    accepted; polygons are fan-triangulated).  Returns a TriangleMesh for the scene graph (-> rtb_scene_set_mesh).
+
+    normals: None = flat facets (the default); "file" = the file's `vn` records through each corner's `/n` index;
+    "smooth" = vertex_normals() of the loaded positions.  uvs=True reads the `vt` records through each corner's `/t`
+    index.  Every stream keeps its own index array, triangulated like the positions; a requested stream that some face
+    lacks raises ValueError.  A negative `scale` mirrors the mesh, so "file" normals are negated with it."""
+    if normals not in (None, "file", "smooth"):
+        raise ValueError('normals must be None, "file" or "smooth"')
     lines = open(path_or_lines).read().splitlines() if isinstance(path_or_lines, str) else list(path_or_lines)
-    verts, tris = [], []
+    verts, vns, vts = [], [], []
+    tris, ntris, ttris = [], [], []
+
+    def ref(tok, count):  # one index of a corner: 1-based, negative = relative to the records read so far
+        i = int(tok)
+        return i - 1 if i > 0 else count + i
+
     for ln in lines:
         p = ln.split()
         if not p or p[0].startswith("#"):
             continue
         if p[0] == "v":
             verts.append([float(p[1]), float(p[2]), float(p[3])])
+        elif p[0] == "vn":
+            vns.append([float(p[1]), float(p[2]), float(p[3])])
+        elif p[0] == "vt":
+            vts.append([float(p[1]), float(p[2]) if len(p) > 2 else 0.0])
         elif p[0] == "f":
-            idx = []
+            idx, nidx, tidx = [], [], []
             for tok in p[1:]:
-                i = int(tok.split("/")[0])
-                idx.append(i - 1 if i > 0 else len(verts) + i)
+                f = tok.split("/")
+                idx.append(ref(f[0], len(verts)))
+                if uvs:
+                    if len(f) < 2 or not f[1]:
+                        raise ValueError(f"OBJ face without texture coordinates: {ln!r}")
+                    tidx.append(ref(f[1], len(vts)))
+                if normals == "file":
+                    if len(f) < 3 or not f[2]:
+                        raise ValueError(f"OBJ face without normals: {ln!r}")
+                    nidx.append(ref(f[2], len(vns)))
             for k in range(1, len(idx) - 1):
                 tris.append([idx[0], idx[k], idx[k + 1]])
+                if nidx:
+                    ntris.append([nidx[0], nidx[k], nidx[k + 1]])
+                if tidx:
+                    ttris.append([tidx[0], tidx[k], tidx[k + 1]])
     v = np.asarray(verts, dtype=np.float64) * scale + np.asarray(offset, dtype=np.float64)
     t = np.asarray(tris, dtype=np.uint32).reshape(-1, 3)
     if len(v) == 0 or len(t) == 0 or t.max() >= len(v):
         raise ValueError("OBJ has no triangles or references a missing vertex")
-    return TriangleMesh(v.astype(np.float32), t, mat)
+    mesh = TriangleMesh(v.astype(np.float32), t, mat)
+    if normals == "file":
+        n = np.asarray(vns, dtype=np.float64).reshape(-1, 3) * (-1.0 if scale < 0 else 1.0)
+        ni = np.asarray(ntris, dtype=np.int64).reshape(-1, 3)
+        if len(n) == 0 or ni.min() < 0 or ni.max() >= len(n):
+            raise ValueError("OBJ face references a missing normal")
+        mesh.normals, mesh.normal_indices = n.astype(np.float32), ni.astype(np.uint32)
+    elif normals == "smooth":
+        mesh.normals = vertex_normals(mesh.vertices, t)
+    if uvs:
+        uv = np.asarray(vts, dtype=np.float64).reshape(-1, 2)
+        ti = np.asarray(ttris, dtype=np.int64).reshape(-1, 3)
+        if len(uv) == 0 or ti.min() < 0 or ti.max() >= len(uv):
+            raise ValueError("OBJ face references a missing texture coordinate")
+        mesh.uvs, mesh.uv_indices = uv.astype(np.float32), ti.astype(np.uint32)
+    return mesh
+
+
+def vertex_normals(vertices, indices) -> np.ndarray:
+    """Smooth-shading normals of an indexed mesh: at each position, the sum of the face normals of the triangles that
+    share it, weighted by their areas (cross(e1, e2) is twice the area times the unit normal), normalised; (n, 3)
+    float32, indexed like the positions.  A position whose faces cancel out gets a zero normal, which the renderer
+    treats as "use the facet normal"."""
+    v = np.asarray(vertices, dtype=np.float64).reshape(-1, 3)
+    t = np.asarray(indices, dtype=np.int64).reshape(-1, 3)
+    fn = np.cross(v[t[:, 1]] - v[t[:, 0]], v[t[:, 2]] - v[t[:, 0]])
+    acc = np.zeros_like(v)
+    for k in range(3):
+        np.add.at(acc, t[:, k], fn)
+    ln = np.linalg.norm(acc, axis=1, keepdims=True)
+    return np.divide(acc, ln, out=np.zeros_like(acc), where=ln > 0).astype(np.float32)
 
 
 def save_image(path: str, rgb8: np.ndarray) -> None:

@@ -130,7 +130,18 @@ class Scene:
             F.check(lib.rtb_scene_set_perlin(self.h, i, F.ptr(rv), F.ptr(px), F.ptr(py), F.ptr(pz)))
         for i, (v, idx) in enumerate(cs.meshes):
             F.check(lib.rtb_scene_set_mesh(self.h, i, F.ptr(v), len(v), F.ptr(idx), len(idx)))
+        for i, attrs in enumerate(cs.mesh_attrs):
+            if attrs is not None:
+                self.set_mesh_attributes(i, *attrs)
         F.check(lib.rtb_scene_set_lights(self.h, F.ptr(cs.lights) if len(cs.lights) else None, len(cs.lights)))
+
+    def set_mesh_attributes(self, mesh_id, normals=None, normal_indices=None, uvs=None, uv_indices=None):
+        """rtb_scene_set_mesh_attributes: vertex normals (k, 3) and / or texture coordinates (j, 2) of a mesh already set,
+        each with an optional (m, 3) index array of its own (None: the mesh's position indices)."""
+        a = lambda x, dt, k: None if x is None else np.ascontiguousarray(x, dtype=dt).reshape(-1, k)
+        n, ni, uv, ui = a(normals, np.float32, 3), a(normal_indices, np.uint32, 3), a(uvs, np.float32, 2), a(uv_indices, np.uint32, 3)
+        F.check(self.lib.rtb_scene_set_mesh_attributes(self.h, mesh_id, F.ptr(n), 0 if n is None else len(n), F.ptr(ni),
+                                                       F.ptr(uv), 0 if uv is None else len(uv), F.ptr(ui)))
 
     def set_compiled(self, cs: CompiledScene):
         self.set_tables(cs)
@@ -180,6 +191,14 @@ class Scene:
                                                     C.byref(ea)))
             out.append(a)
         return out, cm.value, ea.value
+
+    def export_triangle_attributes(self):
+        """(n_triangles, 16) float32 shading records in triangle leaf order (export_bvh's prims[3]); see include/rtb200.h"""
+        n = self.info()["n_triangles"]
+        out = np.zeros((n, 16), dtype=np.float32)
+        if n:
+            F.check(self.lib.rtb_scene_export_triangle_attributes(self.h, F.ptr(out), out.nbytes))
+        return out
 
     def export_globals(self):
         """refs (type << 29 | index) of the primitives that are tested for every ray instead of living in the tree"""

@@ -222,9 +222,16 @@ class Quad(Hittable):  # new: RTTNW quad(Q, u, v)
 
 @dataclass(eq=False)
 class TriangleMesh(Hittable):  # new: indexed mesh (OBJ-style), vertices f32
+    """Optional shading attributes (rtb_scene_set_mesh_attributes): per-vertex `normals` (k, 3) for smooth shading and
+    texture coordinates `uvs` (j, 2), each with its own (m, 3) index array as in OBJ; an index array of None reuses
+    `indices` (the stream then has one entry per vertex)."""
     vertices: np.ndarray  # (n, 3) float32
     indices: np.ndarray   # (m, 3) uint32
     mat: Material
+    normals: Optional[np.ndarray] = None
+    uvs: Optional[np.ndarray] = None
+    normal_indices: Optional[np.ndarray] = None
+    uv_indices: Optional[np.ndarray] = None
 
 
 @dataclass(eq=False)
@@ -300,13 +307,15 @@ class CompiledScene:
     images: list             # [(h,w,3) uint8]
     perlins: list            # [Perlin]
     meshes: list             # [(verts f32 (n,3), idx u32 (m,3))]
+    # per mesh: None, or (normals f32 (k,3) | None, normal idx u32 (m,3) | None, uvs f32 (j,2) | None, uv idx u32 (m,3) | None)
+    mesh_attrs: list = field(default_factory=list)
 
 
 class _Compiler:
     def __init__(self):
         self.nodes, self.children = [], []
         self.materials, self.textures = [], []
-        self.images, self.perlins, self.meshes = [], [], []
+        self.images, self.perlins, self.meshes, self.mesh_attrs = [], [], [], []
         self._mat_ids, self._tex_ids = {}, {}
         self._keep = []  # keeps temporaries alive so id() keys stay unique
 
@@ -384,6 +393,10 @@ class _Compiler:
             p[0] = float(len(self.meshes))
             self.meshes.append((np.ascontiguousarray(h.vertices, dtype=np.float32).reshape(-1, 3),
                                 np.ascontiguousarray(h.indices, dtype=np.uint32).reshape(-1, 3)))
+            a = lambda x, dt, k: None if x is None else np.ascontiguousarray(x, dtype=dt).reshape(-1, k)
+            attrs = (a(h.normals, np.float32, 3), a(h.normal_indices, np.uint32, 3), a(h.uvs, np.float32, 2),
+                     a(h.uv_indices, np.uint32, 3))
+            self.mesh_attrs.append(None if attrs[0] is None and attrs[2] is None else attrs)
         elif isinstance(h, Translate):
             ty = F.NODE_TRANSLATE
             p[0:3] = list(h.offset)
@@ -439,4 +452,4 @@ def compile_scene(world: Hittable, lights: Optional[HittableList] = None) -> Com
     for i, r in enumerate(lrec):
         larr[i] = r
     return CompiledScene(nodes, np.asarray(c.children, dtype=np.uint32), root, mats, texs, larr, c.images, c.perlins,
-                         c.meshes)
+                         c.meshes, c.mesh_attrs)

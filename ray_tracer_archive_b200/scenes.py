@@ -225,7 +225,7 @@ def heightfield_mesh(nx=1000, nz=500, seed=1, x0=65.0, x1=490.0, z0=65.0, z1=490
     return verts, tris
 
 
-def mesh_cornell(nx=1000, nz=500, seed=1) -> HittableList:
+def mesh_cornell(nx=1000, nz=500, seed=1, smooth=False) -> HittableList:
     objects = HittableList.new()
     red = Lambertian.construct((0.65, 0.05, 0.05))
     white = Lambertian.construct((0.73, 0.73, 0.73))
@@ -238,7 +238,8 @@ def mesh_cornell(nx=1000, nz=500, seed=1) -> HittableList:
     objects.add(XzRect.construct(0.0, 555.0, 0.0, 555.0, 555.0, white))
     objects.add(XyRect.construct(0.0, 555.0, 0.0, 555.0, 555.0, white))
     verts, tris = heightfield_mesh(nx, nz, seed)
-    objects.add(TriangleMesh(verts, tris, white))
+    from .io import vertex_normals
+    objects.add(TriangleMesh(verts, tris, white, normals=vertex_normals(verts, tris) if smooth else None))
     return objects
 
 
@@ -248,10 +249,68 @@ def mesh_lights() -> HittableList:
     return lights
 
 
-def config_mesh(width=1920, height=1080, spp=1024, nx=1000, nz=500, seed=1) -> Config:
+def config_mesh(width=1920, height=1080, spp=1024, nx=1000, nz=500, seed=1, smooth=False) -> Config:
+    """smooth=True: the height field carries area-weighted vertex normals (io.vertex_normals) and is shaded smooth."""
     cam = _cam((278.0, 278.0, -800.0), (278.0, 278.0, 0.0), 40.0, width / height, 0.0)
-    return Config(f"C4 {2 * nx * nz}-triangle mesh in a Cornell box", mesh_cornell(nx, nz, seed), mesh_lights(), cam,
-                  width, height, spp, 50, (0.0, 0.0, 0.0))
+    return Config(f"C4 {2 * nx * nz}-triangle {'smooth ' if smooth else ''}mesh in a Cornell box",
+                  mesh_cornell(nx, nz, seed, smooth), mesh_lights(), cam, width, height, spp, 50, (0.0, 0.0, 0.0))
+
+
+def uv_sphere_mesh(center, radius, n_lon, n_lat, mat, uvs=True) -> TriangleMesh:
+    """Latitude-longitude sphere: 2 poles + (n_lat - 1) rings of n_lon positions, shared along the seam, with unit
+    vertex normals on the positions' own indices.  Texture coordinates (sphere.rs:32-37's u = phi / 2pi, v = theta / pi
+    convention) live on their own index stream: the seam has u = 0 on one side and u = 1 on the other, and each pole
+    triangle has its own pole texel column."""
+    c = np.asarray(center, dtype=np.float64)
+    theta = np.pi * np.arange(1, n_lat) / n_lat                  # polar angle from -y (v = theta / pi), rings only
+    phi = 2.0 * np.pi * np.arange(n_lon) / n_lon                 # u = phi / 2pi
+    T, P = np.meshgrid(theta, phi, indexing="ij")
+    # sphere.rs:32-37: theta = acos(-y), phi = atan2(-z, x) + pi  ->  x = -cos(phi) sin(theta), z = sin(phi) sin(theta)
+    ring = np.stack([-np.cos(P) * np.sin(T), -np.cos(T), np.sin(P) * np.sin(T)], -1).reshape(-1, 3)
+    unit = np.concatenate([[[0.0, -1.0, 0.0]], ring, [[0.0, 1.0, 0.0]]])
+    south, north = 0, len(unit) - 1
+    pos = lambda i, j: 1 + i * n_lon + (j % n_lon)               # ring i, longitude j (the seam wraps to j = 0)
+    # texture coordinates: (n_lat - 1) rings of n_lon + 1 (u = 1 duplicates the seam), then one pole texel per column
+    uv_ring = np.stack(np.meshgrid(np.arange(n_lon + 1) / n_lon, theta / np.pi, indexing="xy"), -1).reshape(-1, 2)
+    cols = (np.arange(n_lon) + 0.5) / n_lon
+    uv = np.concatenate([uv_ring, np.stack([cols, np.zeros(n_lon)], 1), np.stack([cols, np.ones(n_lon)], 1)])
+    tuv = lambda i, j: i * (n_lon + 1) + j
+    s_uv, n_uv = (n_lat - 1) * (n_lon + 1), (n_lat - 1) * (n_lon + 1) + n_lon
+    tri, tri_uv = [], []
+    for j in range(n_lon):  # outward-facing winding: cross(e1, e2) points away from the centre
+        tri.append([south, pos(0, j + 1), pos(0, j)]); tri_uv.append([s_uv + j, tuv(0, j + 1), tuv(0, j)])
+        for i in range(n_lat - 2):
+            tri.append([pos(i, j), pos(i, j + 1), pos(i + 1, j + 1)])
+            tri_uv.append([tuv(i, j), tuv(i, j + 1), tuv(i + 1, j + 1)])
+            tri.append([pos(i, j), pos(i + 1, j + 1), pos(i + 1, j)])
+            tri_uv.append([tuv(i, j), tuv(i + 1, j + 1), tuv(i + 1, j)])
+        tri.append([north, pos(n_lat - 2, j), pos(n_lat - 2, j + 1)])
+        tri_uv.append([n_uv + j, tuv(n_lat - 2, j), tuv(n_lat - 2, j + 1)])
+    verts = (c + radius * unit).astype(np.float32)
+    return TriangleMesh(verts, np.asarray(tri, np.uint32), mat, normals=unit.astype(np.float32),
+                        uvs=uv.astype(np.float32) if uvs else None,
+                        uv_indices=np.asarray(tri_uv, np.uint32) if uvs else None)
+
+
+def smooth_meshes(earth_img: Optional[np.ndarray] = None) -> HittableList:
+    """The Cornell box of C4 (walls, light) holding three smooth-shaded meshes: an earthmap-textured UV sphere under
+    RotateY + Translate, a mirror-metal sphere and a glass sphere, both coarse enough that flat facets would show."""
+    objects = HittableList.new()
+    for o in mesh_cornell(1, 1).objects[:6]:  # the walls and the light (the height field is left out)
+        objects.add(o)
+    img = earth_img if earth_img is not None else earthmap()
+    earth_mat = Lambertian.construct_texture(ImageTexture.construct(img, img.shape[1], img.shape[0]))
+    globe = uv_sphere_mesh((0.0, 0.0, 0.0), 110.0, 48, 24, earth_mat)
+    objects.add(Translate.construct(RotateY.construct(globe, 40.0), (390.0, 110.0, 330.0)))
+    objects.add(uv_sphere_mesh((150.0, 90.0, 160.0), 90.0, 16, 8, Metal.construct((0.8, 0.85, 0.88), 0.0), uvs=False))
+    objects.add(uv_sphere_mesh((300.0, 330.0, 150.0), 70.0, 12, 6, Dielectric.construct(1.5), uvs=False))
+    return objects
+
+
+def config_smooth_meshes(width=400, height=400, spp=256) -> Config:
+    cam = _cam((278.0, 278.0, -800.0), (278.0, 278.0, 0.0), 40.0, width / height, 0.0)
+    return Config("smooth-shaded, UV-mapped meshes in a Cornell box", smooth_meshes(), mesh_lights(), cam, width,
+                  height, spp, 50, (0.0, 0.0, 0.0))
 
 
 # ---------------------------------------------------------------------------------------------- small regression scenes
